@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference|reference-gpu]
                     [--api fused|dropin] [--model tv2o-medium|tv2o-large|...] [--events S] [--batch B]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +22,11 @@ Default workload = BASELINE.json configs[1]: tv2o-medium, B=8, S=2048.  Metric: 
   generate     : BASELINE's second metric, events/s of the KV-cached generate loop, with its HBM roofline
   cpu_baseline : the oracle port of the reference's path (fp32 eager PyTorch, host cores) on a
                  bounded sample (B=1, S=128 train step), rank 0 at N=1 only
+
+--dump-outputs DIR (native arm, rank 0) writes what the last timed step computed as DIR/<name>.npy (float32): `loss`, and
+`param.<name>` / `grad.<name>` for every trainable parameter after the optimizer update.  Inputs and weights are seeded, so
+two builds run with the same arguments can be compared output for output -- to a tolerance: the order of the atomic
+gradient accumulations varies, and two runs of one build already differ in the last bits.
 
 Arms:
   --impl native (default)   this repo's kernels.  --api fused = MIDIModel.training_loss + fused_optimizer_step (the
@@ -225,7 +231,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
-    steps, warmup = max(1, min(args.steps, 6)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, max(1, min(args.warmup, 2))
     v, ms, cores, sample = cpu_train_step_tokens_per_s(args.model, steps, warmup)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -433,7 +439,7 @@ def run_native(args):
             return loss
 
     timed = make_timed(world, dev, lambda: lib.query("b200_launch_count"))
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     for i in range(W):
         step(resident[i % n_batches])
     torch.cuda.synchronize()
@@ -441,7 +447,13 @@ def run_native(args):
     sampler = ClockSampler(local)
     sampler.start()
     time.sleep(0.3)
-    ms_total, launches, t0, t1 = timed(lambda i: step(resident[i % n_batches]), K)      # the timed region (`value`)
+    last = {}
+
+    def timed_step(i):
+        last["loss"] = step(resident[i % n_batches])
+    ms_total, launches, t0, t1 = timed(timed_step, K)      # the timed region (`value`)
+    # taken before the passes below run more steps on the same model
+    outputs = last_step_outputs(model, last["loss"]) if args.dump_outputs and rank == 0 else None
     # Roofline pass: the same K steps again with CUDA events around every GEMM launch.  It runs single-stream (the
     # weight-gradient GEMMs of the timed region run on a side stream under the HBM-bound kernels, where an event pair
     # would time the co-running kernels too), so `achieved` is each GEMM's own duration inside a full step.
@@ -526,12 +538,39 @@ def run_native(args):
     if world == 1 and not args.no_cpu_baseline:
         v, ms, cores, sample = cpu_train_step_tokens_per_s(args.model, 3, 1)
         line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample, "ms_per_step": ms}
+    if outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+DUMP_BUDGET_BYTES = 48 << 20
+
+
+def last_step_outputs(model, loss):
+    """The arrays a caller of the timed step holds after it: the loss, and every trainable parameter as the optimizer left
+    it with the gradient that step computed.  A tensor larger than an equal share of DUMP_BUDGET_BYTES is reduced to a
+    fixed, seeded sample of that many elements (the same positions for the parameter and its gradient)."""
+    import numpy as np
+    params = [(n, p) for n, p in model.named_parameters() if p.requires_grad]
+    share = DUMP_BUDGET_BYTES // 4 // (2 * len(params))
+    rng = np.random.default_rng(0)
+    out = {"loss": loss.detach().float().cpu().numpy()}
+    for name, p in params:
+        idx = None
+        if p.numel() > share:
+            idx = torch.from_numpy(np.sort(rng.choice(p.numel(), share, replace=False))).to(p.device)
+        for kind, t in (("param", p), ("grad", p.grad)):
+            flat = t.detach().reshape(-1)
+            out[f"{kind}.{name}"] = (flat if idx is None else flat[idx]).float().cpu().numpy()
+    return out
 
 
 def gemm_traffic():
@@ -701,7 +740,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-generate", action="store_true")
     ap.add_argument("--no-hbm-kernels", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs is implemented for --impl native")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "reference-gpu":

@@ -12,6 +12,9 @@ imported read-only through oracle/ref_loader.py.
               loss on a (1,17,8) synthetic batch (weights regenerated from seed).
   app_stream.npz  events yielded by the reference's app.py generate() (app.py:27-120, executed from the reference
               file at run time, nothing copied) on the tiny model with the disable_* options, greedy and sampled.
+  tokenizer.json  the reference tokenizer's id tables (v1 and v2): every attribute the drop-in mirrors, and to_dict().
+  medium_4layer.npz  the reference's fp32 hidden states (full) and logits (a seeded sample of 256 vocabulary columns,
+              plus the norm of all of them) for a 4-layer model of tv2o-medium width, seed-1 weights, on a (1, 9, 8) batch.
 """
 from __future__ import annotations
 
@@ -165,6 +168,8 @@ APP_CASES = {
     "sampled": dict(prompt="batch4", batch_size=2, max_len=12, temp=1.0, top_p=0.98, top_k=20, disable_patch_change=False,
                     disable_control_change=True, disable_channels=[9], seed=3),
     "plain": dict(prompt="batch4", batch_size=2, max_len=10, top_k=1),
+    "options": dict(prompt=None, batch_size=3, max_len=9, temp=0.9, top_p=0.95, top_k=10, disable_patch_change=True,
+                    disable_control_change=False, disable_channels=[0, 3], seed=21),
 }
 
 
@@ -187,12 +192,47 @@ def app_stream():
     np.savez_compressed(os.path.join(OUT, "app_stream.npz"), **out)
 
 
+TOKENIZER_ATTRS = ("vocab_size", "pad_id", "bos_id", "eos_id", "events", "event_parameters", "event_ids", "parameter_ids",
+                   "max_token_seq")
+
+
+def tokenizer():
+    """id_events is stored as [id, name] pairs: JSON object keys are strings."""
+    import json
+    _, rt = ref_loader.load()
+    out = {}
+    for ver in ("v1", "v2"):
+        t = rt.MIDITokenizer(ver)
+        out[ver] = {a: getattr(t, a) for a in TOKENIZER_ATTRS}
+        out[ver]["id_events"] = sorted([i, e] for i, e in t.id_events.items())
+        out[ver]["to_dict"] = t.to_dict()
+    with open(os.path.join(OUT, "tokenizer.json"), "w") as f:
+        json.dump(out, f, separators=(",", ":"))
+        f.write("\n")
+
+
+MEDIUM_4LAYER_COLS = 256
+
+
+def medium_4layer():
+    mm, _ = ref_loader.load()
+    torch.manual_seed(1)
+    cfg = mm.MIDIModelConfig.get_config("v2", True, n_layer=4, n_head=16, n_embd=1024, n_inner=4096)
+    model = mm.MIDIModel(cfg).eval()
+    batch = synth_batch(model.tokenizer, 1, 9, seed=5)
+    with torch.no_grad():
+        h = model.forward(batch[:, :-1])
+        lg = model.forward_token(h.reshape(-1, 1024), batch[:, 1:].reshape(-1, 8)[:, :-1])
+    cols = np.sort(np.random.default_rng(0).choice(lg.shape[-1], MEDIUM_4LAYER_COLS, replace=False))
+    out = {"batch": batch.numpy(), "fp32/hidden": h.numpy(), "logit_cols": cols, "fp32/logits_sample": lg.numpy()[..., cols],
+           "fp32/logits_norm": np.float64(lg.double().norm().item())}
+    np.savez_compressed(os.path.join(OUT, "medium_4layer.npz"), **out)
+    print("medium_4layer.npz: hidden", tuple(h.shape), "logits", tuple(lg.shape))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
-    if len(sys.argv) > 1 and sys.argv[1] == "app_stream":
-        app_stream()
-    else:
-        tiny()
-        medium()
-        app_stream()
+    steps = {"tiny": tiny, "medium": medium, "app_stream": app_stream, "tokenizer": tokenizer, "medium_4layer": medium_4layer}
+    for name in sys.argv[1:] or steps:
+        steps[name]()

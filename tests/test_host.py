@@ -283,6 +283,41 @@ def test_bench_reference_arm_contract():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_bench_last_step_outputs(monkeypatch):
+    """`bench.py --dump-outputs`: the loss and every trainable parameter with its gradient in float32, within the byte
+    budget; a tensor over its share is sampled at the same seeded positions for parameter and gradient, run after run."""
+    import importlib.util
+    import midi_model as mm
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 1 << 20)
+    torch.manual_seed(0)
+    m = mm.MIDIModel(mm.MIDIModelConfig.get_config("v2", True, n_layer=4, n_head=4, n_embd=32, n_inner=64))
+    named = list(m.named_parameters())
+    for _, p in named:
+        p.grad = -2 * p.detach()
+    out = bench.last_step_outputs(m, torch.tensor(1.5))
+    assert set(out) == {"loss"} | {f"{k}.{n}" for n, _ in named for k in ("param", "grad")}
+    assert out["loss"] == np.float32(1.5)
+    assert all(a.dtype == np.float32 for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= (1 << 20) + 4
+    share = (1 << 20) // 4 // (2 * len(named))
+    sampled = 0
+    for n, p in named:
+        a, g = out["param." + n], out["grad." + n]
+        np.testing.assert_array_equal(g, -2 * a)
+        full = p.detach().reshape(-1).numpy()
+        if p.numel() <= share:
+            np.testing.assert_array_equal(a, full)
+        else:
+            sampled += 1
+            assert a.shape == (share,) and np.isin(a, full).all()
+    assert sampled >= 3                                   # the two embedding tables and lm_head
+    again = bench.last_step_outputs(m, torch.tensor(1.5))
+    assert all(np.array_equal(out[k], again[k]) for k in out)
+
+
 def test_no_cpu_fallback():
     import midi_model as mm
     from midi_b200.lib import B200Error

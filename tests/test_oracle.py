@@ -1,13 +1,16 @@
 """Pin the CPU oracle (oracle/midi_oracle.py) against fixtures produced by the
-unmodified reference (oracle/make_golden.py), and -- when /root/reference is
-present (build container) -- against the reference run live."""
+unmodified reference (oracle/make_golden.py)."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import midi_oracle as O
-from oracle import ref_loader
 from midi_b200.tokenizer_tables import TokenizerTables
+
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 TINY = O.ModelCfg(vocab=3406, n_layer=4, n_head=4, n_embd=32, n_inner=64)
 
@@ -31,15 +34,17 @@ def test_tokenizer_tables_v2():
     assert TokenizerTables("v1").vocab_size == 3239
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference not present")
 def test_tokenizer_tables_match_reference():
-    _, rt = ref_loader.load()
+    """The id tables equal the reference tokenizer's (tests/golden/tokenizer.json, written by oracle/make_golden.py)."""
+    with open(os.path.join(GOLDEN, "tokenizer.json")) as f:
+        ref = json.load(f)
     for ver in ("v1", "v2"):
-        a, b = TokenizerTables(ver), rt.MIDITokenizer(ver)
+        a, b = TokenizerTables(ver), ref[ver]
         for attr in ("vocab_size", "pad_id", "bos_id", "eos_id", "events", "event_parameters", "event_ids",
-                     "id_events", "parameter_ids", "max_token_seq"):
-            assert getattr(a, attr) == getattr(b, attr), attr
-        assert a.to_dict() == b.to_dict()
+                     "parameter_ids", "max_token_seq"):
+            assert getattr(a, attr) == b[attr], attr
+        assert a.id_events == {i: e for i, e in b["id_events"]}
+        assert a.to_dict() == b["to_dict"]
 
 
 def test_forward_fp32_golden(golden_tiny):
@@ -129,8 +134,7 @@ def _app_stream_kwargs(name, g):
 def test_app_stream_golden(golden_tiny, case):
     """oracle.generate_stream (+ deny masks, 4096-event window) == the events the reference's app.py generate() yields
     (tests/golden/app_stream.npz, produced by oracle/make_golden.py from the reference file itself)."""
-    import os
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "app_stream.npz"))
+    g = np.load(os.path.join(GOLDEN, "app_stream.npz"))
     tok, prompt, seed, deny, kw = _app_stream_kwargs(case, g)
     sd = tiny_sd(golden_tiny)
     blocks = list(O.generate_stream(sd, TINY, tok, prompt, generator=torch.Generator().manual_seed(seed), deny=deny,
@@ -144,24 +148,15 @@ def test_app_stream_golden(golden_tiny, case):
         np.testing.assert_array_equal(evs, golden_tiny["gen/greedy_prompt_ids"][:, P:])
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference not present")
 def test_app_stream_vs_live_reference(golden_tiny):
-    """Same comparison against app.py's generate() executed live from /root/reference (build container only)."""
-    from oracle.make_golden import ref_app_generate, APP_CASES
-    mm, _ = ref_loader.load()
-    torch.manual_seed(0)
-    cfg = mm.MIDIModelConfig.get_config("v2", True, n_layer=4, n_head=4, n_embd=32, n_inner=64)
-    model = mm.MIDIModel(cfg).eval()
-    gen = ref_app_generate(model, model.tokenizer)
-    tok = TokenizerTables("v2")
-    kw = dict(batch_size=3, max_len=9, temp=0.9, top_p=0.95, top_k=10, disable_patch_change=True,
-              disable_control_change=False, disable_channels=[0, 3])
-    ref = np.stack(list(gen(prompt=None, generator=torch.Generator().manual_seed(21), **kw)), axis=1)
-    sd = {k: v.detach() for k, v in model.state_dict().items()}
-    deny = O.deny_ids(tok, True, False, [0, 3])
-    blocks = list(O.generate_stream(sd, TINY, tok, None, batch_size=3, max_len=9, temp=0.9, top_p=0.95, top_k=10,
-                                    generator=torch.Generator().manual_seed(21), deny=deny, max_context=4096))
-    np.testing.assert_array_equal(np.stack([b.numpy() for b in blocks[1:]], axis=1), ref)
+    """Three sampled rows with temperature, top-p / top-k, no patch changes and two channels denied == the events
+    app.py's generate() yielded for the same call (the "options" case of tests/golden/app_stream.npz)."""
+    g = np.load(os.path.join(GOLDEN, "app_stream.npz"))
+    tok, prompt, seed, deny, kw = _app_stream_kwargs("options", g)
+    assert prompt is None and deny == O.deny_ids(tok, True, False, [0, 3])
+    blocks = list(O.generate_stream(tiny_sd(golden_tiny), TINY, tok, None, generator=torch.Generator().manual_seed(seed),
+                                    deny=deny, max_context=4096, **kw))
+    np.testing.assert_array_equal(np.stack([b.numpy() for b in blocks[1:]], axis=1), g["options"])
 
 
 def test_sampler_golden(golden_tiny):
@@ -173,21 +168,23 @@ def test_sampler_golden(golden_tiny):
         np.testing.assert_array_equal(s.numpy(), g[f"samp/{name}"])
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference not present")
 def test_oracle_vs_live_reference_medium_shape():
-    """Live cross-check at tv2o-medium width with 2 layers worth of compute kept small:
-    uses the reference's own class on a (1, 9, 8) batch."""
-    mm, _ = ref_loader.load()
+    """Cross-check at tv2o-medium width with the compute kept small (4 layers, a (1, 9, 8) batch) against the reference's
+    own class on the same seed-1 weights, which the drop-in class regenerates bit for bit (tests/golden/medium_4layer.npz:
+    hidden states in full, logits as a seeded column sample plus the norm of all of them)."""
+    import midi_model as mm
+    from midi_b200.synth import synth_batch
+    g = np.load(os.path.join(GOLDEN, "medium_4layer.npz"))
     torch.manual_seed(1)
     cfg = mm.MIDIModelConfig.get_config("v2", True, n_layer=4, n_head=16, n_embd=1024, n_inner=4096)
     model = mm.MIDIModel(cfg).eval()
-    from midi_b200.synth import synth_batch
     batch = synth_batch(model.tokenizer, 1, 9, seed=5)
+    np.testing.assert_array_equal(batch.numpy(), g["batch"])
     sd = {k: v.detach() for k, v in model.state_dict().items()}
     ocfg = O.cfg_from_hf(cfg)
     with torch.no_grad():
-        h_ref = model.forward(batch[:, :-1])
-        l_ref = model.forward_token(h_ref.reshape(-1, 1024), batch[:, 1:].reshape(-1, 8)[:, :-1])
         h = O.forward(sd, ocfg, batch[:, :-1])
         l = O.forward_token(sd, ocfg, h.reshape(-1, 1024), batch[:, 1:].reshape(-1, 8)[:, :-1])
-    assert O.rel_fro(h, h_ref) < 1e-5 and O.rel_fro(l, l_ref) < 1e-5
+    assert O.rel_fro(h, torch.from_numpy(g["fp32/hidden"])) < 1e-5
+    assert O.rel_fro(l[..., torch.from_numpy(g["logit_cols"])], torch.from_numpy(g["fp32/logits_sample"])) < 1e-5
+    assert abs(l.double().norm().item() - float(g["fp32/logits_norm"])) < 1e-5 * float(g["fp32/logits_norm"])
