@@ -123,15 +123,15 @@ int b200_attn_causal_bwd(const void* q, const void* k, const void* v, const void
                          const long long* strides /*8x3: q,k,v,o,do,dq,dk,dv*/, int batch, int n_heads, int Sq, int Sk,
                          int head_dim, float scale, const void* rope_cos /*may be NULL: fuse RoPE backward into dq, dk*/,
                          const void* rope_sin, cudaStream_t s);
-/*      backward on tcgen05 (5 UMMA groups per tile pair, dQ accumulated in fp32 with red.global); training shapes only */
+/*      backward on tcgen05 (5 UMMA groups per tile pair, dQ tiles added into an fp32 accumulator by TMA reduce-add);
+ *      training shapes only */
 size_t b200_attn_causal_bwd_tc_workspace_bytes(int batch, int n_heads, int Sq);
 int b200_attn_causal_bwd_tc(const void* q, const void* k, const void* v, const void* o, const void* d_o, const float* lse,
                             void* dq, void* dk, void* dv, const long long* strides /*8x3: q,k,v,o,do,dq,dk,dv*/, int batch,
                             int n_heads, int Sq, int Sk, int head_dim, float scale, const void* rope_cos /*may be NULL*/,
                             const void* rope_sin, void* workspace, size_t workspace_bytes, cudaStream_t s);
 /*      tuning hook, device buffer of 128 int64 (NULL = off): while set, b200_attn_causal_fwd_tc launches its instrumented
-        instantiation, which adds per-phase clock64 sums of the softmax warps into buf[group*16 + phase] (tools/attn_fwd_profile.py),
-        and the split dQ kernel writes a clock64 trace of CTA (0,0) */
+        instantiation, which adds per-phase clock64 sums of the softmax warps into buf[group*16 + phase] (tools/attn_fwd_profile.py) */
 void b200_attn_debug_trace(long long* buf);
 /*      inner stack: L <= 8 positions per event, head_dim 256, packed qkv rows [n_events*L, ld_qkv]. */
 /*      rope_cos/sin != NULL: qkv holds PRE-RoPE projections; q and k are rotated in place (fused RoPE) before use */

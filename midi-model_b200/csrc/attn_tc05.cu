@@ -2,35 +2,23 @@
 // every matmul is tcgen05.mma with accumulators in TMEM, Q / K / V / dO tiles are staged by TMA (cp.async.bulk.tensor.3d,
 // 128B swizzle, zero fill outside the sequence) straight from the packed [rows, 3*hidden] QKV activation, and the
 // fp32 softmax math runs on dedicated warps that exchange tiles with the MMA-issuing thread(s) through mbarriers.
-// Kernels, in file order (forward generations are selected with B200_ATTN_FWD_TC=v1|v2|v3|v4, default v3):
-//   attn_fwd_tc05_kernel      v1: 4 softmax warps, thread = query row, 2 CTAs/SM
-//   attn_fwd_tc05_v2_kernel   v2: 1 CTA/SM, thread = row x 32 keys, S / P / PV double-buffered, output folded in registers (0.190 ms)
-//   attn_fwd_tc05_v3_kernel   v3 (default): persistent, two query tiles per CTA, thread = row, O in TMEM with a lazy rescale,
-//                             ping-pong between the two softmax groups (0.147-0.155 ms per layer at B=8, S=2048)
-//   attn_fwd_tc05_v4_kernel   v4: v3 with two threads per row (16 softmax warps, setmaxnreg); measured equal to v3, kept as
-//                             the record of that experiment (DESIGN.md 3.1b)
-//   attn_bwd_tc05_kernel<M>   default backward (dK, dV and -- M = 2 -- dQ through a TMA reduce-add), half-tile pipeline
-//   attn_bwd_dq_tc05_kernel   atomic-free dQ for the `split` variant;  attn_bwd_dq_finalize_kernel: fp32 dQ -> bf16
+// Kernels, in file order:
+//   attn_fwd_tc05_kernel         forward: persistent, two query tiles per CTA, thread = row, O in TMEM with a lazy rescale,
+//                                ping-pong between the two softmax groups (0.147-0.155 ms per layer at B=8, S=2048)
+//   attn_bwd_tc05_kernel         backward: dK, dV and dQ (through a TMA reduce-add), half-tile pipeline
+//   attn_bwd_dq_finalize_kernel  fp32 dQ -> bf16
+// DESIGN.md 3.1b has the measurements behind these choices and the variants they ruled out.
 // Semantics = hf sdpa_attention.py:92-101 (causal, scale d^-1/2): online softmax in fp32, P rounded to bf16
 // before P.V, output rounded to bf16, LSE saved for the backward pass.
-#include <cstring>
 #include "tc05.cuh"
 
 namespace {
 using namespace tc05;
 
 constexpr int D = 64;
-constexpr int BQ = 128;    // query rows per CTA
+constexpr int BQ = 128;    // query rows per tile
 constexpr int BK = 128;    // keys per tile
-constexpr int KV_STAGES = 2;
-constexpr int NTHREADS = 192;
 constexpr float LOG2E = 1.4426950408889634f;
-
-constexpr int SM_Q = 0;                                  // 16 KB
-constexpr int SM_KV = 16384;                             // KV_STAGES x (K 16 KB + V 16 KB)
-constexpr int SM_P = SM_KV + KV_STAGES * 32768;          // 32 KB: two 64-key atoms of [128 rows x 128 B]
-constexpr int SM_BAR = SM_P + 32768;
-constexpr int SMEM_BYTES = SM_BAR + 128;
 
 __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1, int c2) {
     asm volatile(
@@ -52,424 +40,11 @@ struct FwdParams {
     int n_heads, Sq, Sk, H;      // H = columns between the q, k and v thirds when packed (used for TMA column coords)
     int q_col0, k_col0, v_col0;  // first column of head 0 in each tensor map
     float scale;
-    long long* dbg;              // forward v3 phase profile (NULL = off)
+    long long* dbg;              // forward phase profile (NULL = off)
 };
 
-__global__ void __launch_bounds__(NTHREADS, 2)
-attn_fwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                     const __grid_constant__ CUtensorMap tmV, const FwdParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BAR);
-    uint64_t* q_full = bars + 0;
-    uint64_t* kv_full = bars + 1;     // [2]
-    uint64_t* kv_empty = bars + 3;    // [2]
-    uint64_t* s_full = bars + 5;
-    uint64_t* s_empty = bars + 6;
-    uint64_t* p_full = bars + 7;
-    uint64_t* pv_full = bars + 8;
-    uint64_t* pv_empty = bars + 9;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 10);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int qt = gridDim.y - 1 - blockIdx.y;     // long (late) tiles first
-    const int bh = blockIdx.x;
-    const int b = bh / p.n_heads, h = bh % p.n_heads;
-    const int q0 = qt * BQ;
-    const int off = p.Sk - p.Sq;
-    int n_kv = min((p.Sk + BK - 1) / BK, (q0 + BQ - 1 + off) / BK + 1);
-    if (n_kv < 1) n_kv = 1;
-
-    if (warp == 0 && lane == 0) {
-        prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV);
-        mbar_init(q_full, 1);
-        for (int s = 0; s < KV_STAGES; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 1); }
-        mbar_init(s_full, 1); mbar_init(s_empty, 4); mbar_init(p_full, 4); mbar_init(pv_full, 1); mbar_init(pv_empty, 4);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(tmem_slot, 256);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tS = tmem_base, tPV = tmem_base + 128;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_expect_tx(q_full, BQ * D * 2);
-            tma_load_3d(smem + SM_Q, &tmQ, q_full, p.q_col0 + h * D, q0, b);
-            int stage = 0; uint32_t phase = 0;
-            for (int j = 0; j < n_kv; j++) {
-                mbar_wait(&kv_empty[stage], phase ^ 1);
-                uint8_t* sK = smem + SM_KV + stage * 32768;
-                mbar_expect_tx(&kv_full[stage], 2 * BK * D * 2);
-                tma_load_3d(sK, &tmK, &kv_full[stage], p.k_col0 + h * D, j * BK, b);
-                tma_load_3d(sK + 16384, &tmV, &kv_full[stage], p.v_col0 + h * D, j * BK, b);
-                if (++stage == KV_STAGES) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            constexpr uint32_t idesc_s = make_idesc(BQ, BK, false, false);    // S[128 x 128] = Q . K^T
-            constexpr uint32_t idesc_pv = make_idesc(BQ, D, false, true);     // PV[128 x 64] = P . V (V is [keys, d]: MN-major B)
-            const uint32_t sQ = smem_u32(smem + SM_Q), sP = smem_u32(smem + SM_P);
-            mbar_wait(q_full, 0);
-            int stage = 0; uint32_t kv_phase = 0, ph = 0;
-            const uint64_t dQ0 = make_smem_desc(sQ, 16, 1024), dP0 = make_smem_desc(sP, 16, 1024);
-            auto issue_s = [&](int st) {
-                const uint64_t dK0 = make_smem_desc(smem_u32(smem + SM_KV + st * 32768), 16, 1024);
-                tc_fence_after();
-#pragma unroll
-                for (int k = 0; k < D / 16; k++)
-                    umma_f16(tS, desc_adv(dQ0, k * 32), desc_adv(dK0, k * 32), idesc_s, k > 0);
-                umma_commit(s_full);
-            };
-            mbar_wait(&kv_full[0], 0);
-            issue_s(0);
-            for (int j = 0; j < n_kv; j++) {
-                const int st_j = stage;
-                const uint64_t dV0 = make_smem_desc(smem_u32(smem + SM_KV + st_j * 32768 + 16384), 16384, 1024);
-                mbar_wait(p_full, ph);            // softmax wrote P_j (and has finished reading S_j)
-                if (++stage == KV_STAGES) { stage = 0; kv_phase ^= 1; }
-                if (j + 1 < n_kv) {               // S_{j+1} goes first so the softmax warps never wait for the tensor pipe
-                    mbar_wait(&kv_full[stage], kv_phase);
-                    issue_s(stage);
-                }
-                mbar_wait(pv_empty, ph ^ 1);      // previous PV tile drained from TMEM
-                tc_fence_after();
-#pragma unroll
-                for (int kk = 0; kk < BK / 16; kk++)
-                    umma_f16(tPV, desc_adv(dP0, (kk >> 2) * 16384 + (kk & 3) * 32), desc_adv(dV0, kk * 2048), idesc_pv, kk > 0);
-                umma_commit(pv_full);
-                umma_commit(&kv_empty[st_j]);
-                ph ^= 1;
-            }
-        }
-    } else {
-        const int quarter = warp & 3;
-        const int row_t = quarter * 32 + lane;            // row inside the tile == TMEM lane
-        const int row = q0 + row_t;
-        const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        const float sl2 = p.scale * LOG2E;
-        float m_i = -INFINITY, l_i = 0.f;
-        float o[D];
-#pragma unroll
-        for (int i = 0; i < D; i++) o[i] = 0.f;
-        uint8_t* sP = smem + SM_P;
-        uint32_t ph = 0;
-        for (int j = 0; j < n_kv; j++) {
-            const int k0 = j * BK;
-            const bool need_mask = (k0 + BK - 1 > q0 + off) || (k0 + BK > p.Sk);
-            mbar_wait(s_full, ph);
-            tc_fence_after();
-            // pass 1: row maximum
-            float mx = m_i;
-#pragma unroll 1
-            for (int c = 0; c < BK / 32; c++) {
-                uint32_t r[32];
-                tmem_ld32(tS + lane_addr + c * 32, r);
-                tmem_ld_wait();
-#pragma unroll
-                for (int i = 0; i < 32; i++) {
-                    float s = __uint_as_float(r[i]);
-                    if (need_mask) {
-                        const int key = k0 + c * 32 + i;
-                        if (key > row + off || key >= p.Sk) s = -INFINITY;
-                    }
-                    mx = fmaxf(mx, s);
-                }
-            }
-            const float msc = (mx == -INFINITY) ? 0.f : mx * sl2;
-            const float alpha = (m_i == -INFINITY) ? 0.f : exp2f(m_i * sl2 - msc);
-            m_i = mx;
-            // pass 2: probabilities -> bf16 -> swizzled P tile in shared memory
-            float rs = 0.f;
-#pragma unroll 1
-            for (int c = 0; c < BK / 32; c++) {
-                uint32_t r[32];
-                tmem_ld32(tS + lane_addr + c * 32, r);
-                tmem_ld_wait();
-                uint32_t pk[16];
-#pragma unroll
-                for (int i = 0; i < 32; i += 2) {
-                    float s0 = __uint_as_float(r[i]), s1 = __uint_as_float(r[i + 1]);
-                    if (need_mask) {
-                        const int key = k0 + c * 32 + i;
-                        if (key > row + off || key >= p.Sk) s0 = -INFINITY;
-                        if (key + 1 > row + off || key + 1 >= p.Sk) s1 = -INFINITY;
-                    }
-                    const float p0 = ex2_approx(fmaf(s0, sl2, -msc)), p1 = ex2_approx(fmaf(s1, sl2, -msc));
-                    rs += p0 + p1;
-                    pk[i >> 1] = pack2(p0, p1);
-                }
-                // keys c*32 .. c*32+31 of this row: atom (c >> 1), 16-byte chunks (c & 1) * 4 .. + 3
-                uint8_t* rowp = sP + (c >> 1) * 16384 + row_t * 128;
-#pragma unroll
-                for (int v = 0; v < 4; v++) {
-                    const int chunk = (c & 1) * 4 + v;
-                    *reinterpret_cast<uint4*>(rowp + ((chunk ^ (row_t & 7)) << 4)) =
-                        make_uint4(pk[4 * v], pk[4 * v + 1], pk[4 * v + 2], pk[4 * v + 3]);
-                }
-            }
-            l_i = l_i * alpha + rs;
-            tc_fence_before();
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) { mbar_arrive(s_empty); mbar_arrive(p_full); }
-            // correction + accumulate this tile's P.V
-            mbar_wait(pv_full, ph);
-            tc_fence_after();
-#pragma unroll
-            for (int c = 0; c < D / 32; c++) {
-                uint32_t r[32];
-                tmem_ld32(tPV + lane_addr + c * 32, r);
-                tmem_ld_wait();
-#pragma unroll
-                for (int i = 0; i < 32; i++) o[c * 32 + i] = o[c * 32 + i] * alpha + __uint_as_float(r[i]);
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(pv_empty);
-            ph ^= 1;
-        }
-        if (row < p.Sq) {
-            const float inv = l_i > 0.f ? 1.f / l_i : 0.f;
-            bf16* dst = p.o + b * p.o_b + (long long)row * p.o_r + h * D;
-#pragma unroll
-            for (int v = 0; v < D / 8; v++) {
-                float f[8];
-#pragma unroll
-                for (int i = 0; i < 8; i++) f[i] = o[v * 8 + i] * inv;
-                *reinterpret_cast<uint4*>(dst + v * 8) = pack8(f);
-            }
-            if (p.lse) p.lse[((long long)b * p.n_heads + h) * p.Sq + row] = m_i * p.scale + logf(l_i);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 256);
-    }
-}
-
-
 // ---------------------------------------------------------------------------------------------
-// forward, second generation: one CTA per SM, 16 softmax warps (thread = query row x 32 of the 128 keys of a tile),
-// S double-buffered in TMEM so the tensor pipe runs one tile ahead of the math, P double-buffered in shared memory,
-// P.V tiles double-buffered in TMEM and folded into register accumulators one tile late.  Only the row maximum is
-// exchanged between the four column slices of a row (4 KB of shared memory, one 128-thread named barrier per tile);
-// row sums stay per-slice until the end.
-// ---------------------------------------------------------------------------------------------
-constexpr int F2_CWARPS = 16;
-constexpr int F2_THREADS = 64 + 32 * F2_CWARPS;
-constexpr int F2_KVS = 4;                                 // K/V stages: S runs two tiles ahead of P.V, TMA latency needs one more
-constexpr int F2_Q = 0;                                   // 16 KB
-constexpr int F2_KV = 16384;                              // F2_KVS x (K 16 KB + V 16 KB)
-constexpr int F2_P = F2_KV + F2_KVS * 32768;              // 2 x 32 KB
-constexpr int F2_MX = F2_P + 2 * 32768;                   // float [2][4][128] row-max exchange, then [4][128] row sums
-constexpr int F2_BAR = F2_MX + 4096;
-constexpr int F2_SMEM = F2_BAR + 256;
-
-__global__ void __launch_bounds__(F2_THREADS, 1)
-attn_fwd_tc05_v2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                        const __grid_constant__ CUtensorMap tmV, const FwdParams p) {
-    B200_PDL_TRIGGER();
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + F2_BAR);
-    uint64_t* q_full = bars + 0;
-    uint64_t* kv_full = bars + 1;     // [F2_KVS]
-    uint64_t* kv_empty = bars + 5;    // [F2_KVS]
-    uint64_t* s_full = bars + 9;      // [2]
-    uint64_t* p_full = bars + 11;     // [2]
-    uint64_t* pv_full = bars + 13;    // [2]
-    uint64_t* pv_empty = bars + 15;   // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 17);
-    float* mx_s = reinterpret_cast<float*>(smem + F2_MX);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int qt = gridDim.y - 1 - blockIdx.y;     // long (late) tiles first
-    const int bh = blockIdx.x;
-    const int b = bh / p.n_heads, h = bh % p.n_heads;
-    const int q0 = qt * BQ;
-    const int off = p.Sk - p.Sq;
-    int n_kv = min((p.Sk + BK - 1) / BK, (q0 + BQ - 1 + off) / BK + 1);
-    if (n_kv < 1) n_kv = 1;
-
-    if (warp == 0 && lane == 0) {
-        prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV);
-        mbar_init(q_full, 1);
-        for (int s = 0; s < F2_KVS; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 1); }
-        for (int s = 0; s < 2; s++) {
-            mbar_init(&s_full[s], 1); mbar_init(&p_full[s], F2_CWARPS); mbar_init(&pv_full[s], 1); mbar_init(&pv_empty[s], F2_CWARPS);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(tmem_slot, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tS = tmem_base /* 2 x 128 columns */, tPV = tmem_base + 256 /* 2 x 64 columns */;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_expect_tx(q_full, BQ * D * 2);
-            tma_load_3d(smem + F2_Q, &tmQ, q_full, p.q_col0 + h * D, q0, b);
-            int stage = 0; uint32_t phase = 0;
-            for (int j = 0; j < n_kv; j++) {
-                mbar_wait(&kv_empty[stage], phase ^ 1);
-                uint8_t* sK = smem + F2_KV + stage * 32768;
-                mbar_expect_tx(&kv_full[stage], 2 * BK * D * 2);
-                tma_load_3d(sK, &tmK, &kv_full[stage], p.k_col0 + h * D, j * BK, b);
-                tma_load_3d(sK + 16384, &tmV, &kv_full[stage], p.v_col0 + h * D, j * BK, b);
-                if (++stage == F2_KVS) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            constexpr uint32_t idesc_s = make_idesc(BQ, BK, false, false);    // S[128 x 128] = Q . K^T
-            constexpr uint32_t idesc_pv = make_idesc(BQ, D, false, true);     // PV[128 x 64] = P . V (V is [keys, d]: MN-major B)
-            const uint32_t sQ = smem_u32(smem + F2_Q), sP = smem_u32(smem + F2_P);
-            mbar_wait(q_full, 0);
-            const uint64_t dQ0 = make_smem_desc(sQ, 16, 1024);
-            auto issue_s = [&](int j) {
-                const int st = j % F2_KVS;
-                mbar_wait(&kv_full[st], (uint32_t)((j / F2_KVS) & 1));
-                const uint64_t dK0 = make_smem_desc(smem_u32(smem + F2_KV + st * 32768), 16, 1024);
-                tc_fence_after();
-#pragma unroll
-                for (int k = 0; k < D / 16; k++)
-                    umma_f16(tS + (j & 1) * 128, desc_adv(dQ0, k * 32), desc_adv(dK0, k * 32), idesc_s, k > 0);
-                umma_commit(&s_full[j & 1]);
-            };
-            issue_s(0);
-            if (n_kv > 1) issue_s(1);
-            for (int j = 0; j < n_kv; j++) {
-                const int bb = j & 1, st = j % F2_KVS;
-                const uint32_t par = (uint32_t)((j >> 1) & 1);
-                const uint64_t dP0 = make_smem_desc(sP + bb * 32768, 16, 1024);
-                const uint64_t dV0 = make_smem_desc(smem_u32(smem + F2_KV + st * 32768 + 16384), 16384, 1024);
-                mbar_wait(&p_full[bb], par);          // P_j written, S_j consumed
-                mbar_wait(&pv_empty[bb], par ^ 1);    // P.V tile j-2 folded into the register accumulators
-                tc_fence_after();
-#pragma unroll
-                for (int kk = 0; kk < BK / 16; kk++)
-                    umma_f16(tPV + bb * 64, desc_adv(dP0, (kk >> 2) * 16384 + (kk & 3) * 32), desc_adv(dV0, kk * 2048), idesc_pv, kk > 0);
-                umma_commit(&pv_full[bb]);
-                umma_commit(&kv_empty[st]);
-                if (j + 2 < n_kv) issue_s(j + 2);     // into the S buffer the math warps have just released
-            }
-        }
-    } else {
-        const int cw = warp - 2;
-        const int quarter = warp & 3;
-        const int cg = cw >> 2;                           // key slice: columns cg*32 .. +31 of the tile; d slice cg*16 .. +15 of P.V
-        const int row_t = quarter * 32 + lane;            // row inside the tile == TMEM lane
-        const int row = q0 + row_t;
-        const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        const float sl2 = p.scale * LOG2E;
-        float m_i = -INFINITY, l_part = 0.f, alpha_prev = 0.f;
-        float o[16];
-#pragma unroll
-        for (int i = 0; i < 16; i++) o[i] = 0.f;
-        auto fold_pv = [&](int j, float alpha) {          // o = o * alpha_j + (P.V)_j for this thread's 16 columns
-            const int bb = j & 1;
-            mbar_wait(&pv_full[bb], (uint32_t)((j >> 1) & 1));
-            tc_fence_after();
-            uint32_t r[16];
-            tmem_ld16(tPV + bb * 64 + lane_addr + cg * 16, r);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; i++) o[i] = fmaf(o[i], alpha, __uint_as_float(r[i]));
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&pv_empty[bb]);
-        };
-        for (int j = 0; j < n_kv; j++) {
-            const int k0 = j * BK, bb = j & 1;
-            const bool need_mask = (k0 + BK - 1 > q0 + off) || (k0 + BK > p.Sk);
-            mbar_wait(&s_full[bb], (uint32_t)((j >> 1) & 1));
-            tc_fence_after();
-            float sv[32];
-            {
-                uint32_t r[32];
-                tmem_ld32(tS + bb * 128 + lane_addr + cg * 32, r);
-                tmem_ld_wait();
-                if (need_mask) {      // diagonal / ragged tiles only: a real (warp-uniform) branch, not predication
-                    const int lim = min(row + off, p.Sk - 1) - (k0 + cg * 32);     // last visible column of this slice
-#pragma unroll
-                    for (int i = 0; i < 32; i++) sv[i] = (i > lim) ? -INFINITY : __uint_as_float(r[i]);
-                    asm volatile("" ::: "memory");
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 32; i++) sv[i] = __uint_as_float(r[i]);
-                }
-            }
-            float mx4[4] = {sv[0], sv[1], sv[2], sv[3]};
-#pragma unroll
-            for (int i = 4; i < 32; i++) mx4[i & 3] = fmaxf(mx4[i & 3], sv[i]);
-            float* mxp = mx_s + bb * 512 + row_t;
-            mxp[cg * 128] = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-            asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");     // the four slices of this row quarter
-            const float mx = fmaxf(fmaxf(m_i, fmaxf(mxp[0], mxp[128])), fmaxf(mxp[256], mxp[384]));
-            const float msc = (mx == -INFINITY) ? 0.f : mx * sl2;
-            const float alpha = (m_i == -INFINITY) ? 0.f : exp2f(m_i * sl2 - msc);
-            m_i = mx;
-            uint32_t pk[16];
-            float rs4[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-                const float p0 = ex2_approx(fmaf(sv[i], sl2, -msc)), p1 = ex2_approx(fmaf(sv[i + 1], sl2, -msc));
-                rs4[(i >> 1) & 3] += p0 + p1;
-                pk[i >> 1] = pack2(p0, p1);
-            }
-            l_part = fmaf(l_part, alpha, (rs4[0] + rs4[1]) + (rs4[2] + rs4[3]));
-            // keys cg*32 .. +31 of this row: atom (cg >> 1), 16-byte chunks (cg & 1) * 4 .. + 3.  Buffer bb was last read by
-            // the P.V MMAs of tile j-2, whose completion this thread saw in fold_pv(j-2) during tile j-1.
-            uint8_t* rowp = smem + F2_P + bb * 32768 + (cg >> 1) * 16384 + row_t * 128;
-#pragma unroll
-            for (int v = 0; v < 4; v++) {
-                const int chunk = (cg & 1) * 4 + v;
-                *reinterpret_cast<uint4*>(rowp + ((chunk ^ (row_t & 7)) << 4)) =
-                    make_uint4(pk[4 * v], pk[4 * v + 1], pk[4 * v + 2], pk[4 * v + 3]);
-            }
-            tc_fence_before();
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&p_full[bb]);
-            if (j > 0) fold_pv(j - 1, alpha_prev);
-            alpha_prev = alpha;
-        }
-        fold_pv(n_kv - 1, alpha_prev);
-        // total row sum: the four slices of a row meet in shared memory
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");         // everyone is done with mx_s
-        mx_s[cg * 128 + row_t] = l_part;
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");
-        const float l_i = (mx_s[row_t] + mx_s[128 + row_t]) + (mx_s[256 + row_t] + mx_s[384 + row_t]);
-        if (row < p.Sq) {
-            const float inv = l_i > 0.f ? 1.f / l_i : 0.f;
-            bf16* dst = p.o + b * p.o_b + (long long)row * p.o_r + h * D + cg * 16;
-#pragma unroll
-            for (int v = 0; v < 2; v++) {
-                float f[8];
-#pragma unroll
-                for (int i = 0; i < 8; i++) f[i] = o[v * 8 + i] * inv;
-                *reinterpret_cast<uint4*>(dst + v * 8) = pack8(f);
-            }
-            if (p.lse && cg == 0) p.lse[((long long)b * p.n_heads + h) * p.Sq + row] = m_i * p.scale + logf(l_i);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// forward, third generation (default): persistent, two query tiles per CTA, thread = one query row.
+// forward: persistent, two query tiles per CTA, thread = one query row.
 //   * grid = one CTA per SM; every CTA walks a static, length-balanced list of work items (snake order over the items sorted
 //     longest first).  An item = two adjacent 128-row query tiles of one (batch, head); both tiles consume the same K/V
 //     stream, so every K/V tile is staged once for 256 query rows.
@@ -482,23 +57,26 @@ attn_fwd_tc05_v2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
 //     are at most 256, exact in fp32 and harmless in bf16), which in practice happens on the first tiles of a row only.
 //   * one MMA-issuing warp per group: S_{j+1} = Q.K^T is issued as soon as the group has read S_j out of TMEM, P.V_j when
 //     P_j is in shared memory.  K/V stages are released when both groups' MMAs on them have retired.
+//   * ping-pong: the two softmax warps that share an SM sub-partition (same row quarter, different group) take turns in the
+//     MUFU-bound half of a tile (pass 2) through a pair of 64-thread named barriers, so that one warp's exponentials run
+//     against the other's tile-load / row-maximum / barrier work instead of against its exponentials.
 //   warp 0: TMA producer   warps 1, 2: MMA issuers of group 0 / 1   warp 3: TMEM allocator   warps 4..7 / 8..11: softmax
 // ---------------------------------------------------------------------------------------------
-constexpr int F3_THREADS = 384;
-constexpr int F3_KVS = 4;                                 // K/V stages
-constexpr int F3_Q = 0;                                   // 2 x 16 KB
-constexpr int F3_P = 32768;                               // 2 x 32 KB (one P tile per group)
-constexpr int F3_KV = F3_P + 2 * 32768;                   // F3_KVS x (K 16 KB + V 16 KB)
-constexpr int F3_BAR = F3_KV + F3_KVS * 32768;
-constexpr int F3_SMEM = F3_BAR + 256;
-constexpr float F3_RESCALE_LOG2 = 8.f;
+constexpr int FWD_THREADS = 384;
+constexpr int FWD_KVS = 4;                               // K/V stages
+constexpr int SF_Q = 0;                                  // 2 x 16 KB
+constexpr int SF_P = 32768;                              // 2 x 32 KB (one P tile per group)
+constexpr int SF_KV = SF_P + 2 * 32768;                  // FWD_KVS x (K 16 KB + V 16 KB)
+constexpr int SF_BAR = SF_KV + FWD_KVS * 32768;
+constexpr int SMEM_FWD_BYTES = SF_BAR + 256;
+constexpr float RESCALE_LOG2 = 8.f;
 
-struct F3Item {
+struct FwdItem {
     int b, h;
     int q0[2], n[2], nt;      // first query row and number of K/V tiles of each group (0 = group idle), max of the two
 };
 
-__device__ __forceinline__ bool f3_item(const FwdParams& p, int round, F3Item& it) {
+__device__ __forceinline__ bool fwd_item(const FwdParams& p, int round, FwdItem& it) {
     const int n_qt = (p.Sq + BQ - 1) / BQ, n_pairs = (n_qt + 1) >> 1;
     const int n_bh = p.batch * p.n_heads;
     const int G = gridDim.x, c = blockIdx.x;
@@ -524,18 +102,16 @@ __device__ __forceinline__ bool f3_item(const FwdParams& p, int round, F3Item& i
     return true;
 }
 
-// PINGPONG: the two softmax warps that share an SM sub-partition (same row quarter, different group) take turns in the
-// MUFU-bound half of a tile (pass 2) through a pair of 64-thread named barriers, so that one warp's exponentials run
-// against the other's tile-load / row-maximum / barrier work instead of against its exponentials.
-template <bool PINGPONG, bool PROF>
-__global__ void __launch_bounds__(F3_THREADS, 1)
-attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                        const __grid_constant__ CUtensorMap tmV, const FwdParams p) {
+// PROF: per-phase clock64 sums of the softmax warps into p.dbg (tools/attn_fwd_profile.py through b200_attn_debug_trace)
+template <bool PROF>
+__global__ void __launch_bounds__(FWD_THREADS, 1)
+attn_fwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
+                     const __grid_constant__ CUtensorMap tmV, const FwdParams p) {
     B200_PDL_TRIGGER();
     extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + F3_BAR);
-    uint64_t* kv_full = bars + 0;      // [F3_KVS]
-    uint64_t* kv_empty = bars + 4;     // [F3_KVS]  one arrival per MMA warp
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SF_BAR);
+    uint64_t* kv_full = bars + 0;      // [FWD_KVS]
+    uint64_t* kv_empty = bars + 4;     // [FWD_KVS]  one arrival per MMA warp
     uint64_t* q_full = bars + 8;       // [2]
     uint64_t* q_empty = bars + 10;     // [2]
     uint64_t* s_full = bars + 12;      // [2]
@@ -549,7 +125,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
 
     if (warp == 0 && lane == 0) {
         prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV);
-        for (int s = 0; s < F3_KVS; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 2); }
+        for (int s = 0; s < FWD_KVS; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 2); }
         for (int g = 0; g < 2; g++) {
             mbar_init(&q_full[g], 1); mbar_init(&q_empty[g], 1); mbar_init(&s_full[g], 1); mbar_init(&s_empty[g], 4);
             mbar_init(&p_full[g], 4); mbar_init(&pv_done[g], 1);
@@ -565,21 +141,21 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
     if (warp == 0) {
         if (lane == 0) {
             uint32_t T = 0, cq[2] = {0, 0};
-            F3Item it;
+            FwdItem it;
             for (int r = 0; r < n_rounds; r++) {
-                if (!f3_item(p, r, it)) continue;
+                if (!fwd_item(p, r, it)) continue;
 #pragma unroll
                 for (int g = 0; g < 2; g++) {
                     if (it.n[g] == 0) continue;
                     mbar_wait(&q_empty[g], (cq[g] & 1) ^ 1);
                     mbar_expect_tx(&q_full[g], BQ * D * 2);
-                    tma_load_3d(smem + F3_Q + g * 16384, &tmQ, &q_full[g], p.q_col0 + it.h * D, it.q0[g], it.b);
+                    tma_load_3d(smem + SF_Q + g * 16384, &tmQ, &q_full[g], p.q_col0 + it.h * D, it.q0[g], it.b);
                     cq[g]++;
                 }
                 for (int j = 0; j < it.nt; j++, T++) {
-                    const int st = T % F3_KVS;
-                    mbar_wait(&kv_empty[st], ((T / F3_KVS) & 1) ^ 1);
-                    uint8_t* sK = smem + F3_KV + st * 32768;
+                    const int st = T % FWD_KVS;
+                    mbar_wait(&kv_empty[st], ((T / FWD_KVS) & 1) ^ 1);
+                    uint8_t* sK = smem + SF_KV + st * 32768;
                     mbar_expect_tx(&kv_full[st], 2 * BK * D * 2);
                     tma_load_3d(sK, &tmK, &kv_full[st], p.k_col0 + it.h * D, j * BK, it.b);
                     tma_load_3d(sK + 16384, &tmV, &kv_full[st], p.v_col0 + it.h * D, j * BK, it.b);
@@ -592,25 +168,25 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
             constexpr uint32_t idesc_s = make_idesc(BQ, BK, false, false);    // S[128 x 128] = Q . K^T
             constexpr uint32_t idesc_pv = make_idesc(BQ, D, false, true);     // O[128 x 64] += P . V (V is [keys, d]: MN-major B)
             const uint32_t tS = tmem_base + g * 128, tO = tmem_base + 256 + g * 64;
-            const uint64_t dQ0 = make_smem_desc(smem_u32(smem + F3_Q + g * 16384), 16, 1024);
-            const uint64_t dP0 = make_smem_desc(smem_u32(smem + F3_P + g * 32768), 16, 1024);
+            const uint64_t dQ0 = make_smem_desc(smem_u32(smem + SF_Q + g * 16384), 16, 1024);
+            const uint64_t dP0 = make_smem_desc(smem_u32(smem + SF_P + g * 32768), 16, 1024);
             uint32_t T = 0, tg = 0, cq = 0;
             auto issue_s = [&](uint32_t Tj) {               // S = Q . K_j^T of the K/V tile with running index Tj
-                const int st = Tj % F3_KVS;
-                mbar_wait(&kv_full[st], (Tj / F3_KVS) & 1);
-                const uint64_t dK0 = make_smem_desc(smem_u32(smem + F3_KV + st * 32768), 16, 1024);
+                const int st = Tj % FWD_KVS;
+                mbar_wait(&kv_full[st], (Tj / FWD_KVS) & 1);
+                const uint64_t dK0 = make_smem_desc(smem_u32(smem + SF_KV + st * 32768), 16, 1024);
                 tc_fence_after();
 #pragma unroll
                 for (int k = 0; k < D / 16; k++) umma_f16(tS, desc_adv(dQ0, k * 32), desc_adv(dK0, k * 32), idesc_s, k > 0);
                 umma_commit(&s_full[g]);
             };
-            F3Item it;
+            FwdItem it;
             for (int r = 0; r < n_rounds; r++) {
-                if (!f3_item(p, r, it)) continue;
+                if (!fwd_item(p, r, it)) continue;
                 const int n = g ? it.n[1] : it.n[0];
                 if (n > 0) { mbar_wait(&q_full[g], cq & 1); cq++; }
                 for (int j = 0; j < it.nt; j++, T++) {
-                    const int st = T % F3_KVS;
+                    const int st = T % FWD_KVS;
                     if (j < n) {
                         if (j == 0) {
                             if (tg > 0) mbar_wait(&s_empty[g], (tg - 1) & 1);      // last tile of the previous item read out
@@ -624,7 +200,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
                         }
                         mbar_wait(&p_full[g], tg & 1);
                         tc_fence_after();
-                        const uint64_t dV0 = make_smem_desc(smem_u32(smem + F3_KV + st * 32768 + 16384), 16384, 1024);
+                        const uint64_t dV0 = make_smem_desc(smem_u32(smem + SF_KV + st * 32768 + 16384), 16384, 1024);
 #pragma unroll
                         for (int kk = 0; kk < BK / 16; kk++)
                             umma_f16(tO, desc_adv(dP0, (kk >> 2) * 16384 + (kk & 3) * 32), desc_adv(dV0, kk * 2048), idesc_pv,
@@ -633,7 +209,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
                         umma_commit(&kv_empty[st]);
                         tg++;
                     } else {
-                        mbar_wait(&kv_full[st], (T / F3_KVS) & 1);                 // the other group's tile: just pass the stage on
+                        mbar_wait(&kv_full[st], (T / FWD_KVS) & 1);                 // the other group's tile: just pass the stage on
                         mbar_arrive(&kv_empty[st]);
                     }
                 }
@@ -647,29 +223,27 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
         const uint32_t tS = tmem_base + g * 128 + lane_addr, tO = tmem_base + 256 + g * 64 + lane_addr;
         const float sl2 = p.scale * LOG2E;
         const int off = p.Sk - p.Sq;
-        uint8_t* sP = smem + F3_P + g * 32768;
+        uint8_t* sP = smem + SF_P + g * 32768;
         uint32_t tg = 0;
         // ping-pong token of this sub-partition: barrier 1 + 2*quarter + g is the one this warp waits on
         const int bar_mine = 1 + 2 * quarter + g, bar_other = 1 + 2 * quarter + (g ^ 1);
-        if (PINGPONG && g == 1) asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");    // group 0 goes first
+        if (g == 1) asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");    // group 0 goes first
         long long pf[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pt = 0;      // PROF: cycles per phase (lane 0), tiles
         const long long pstart = PROF ? clock64() : 0;
         auto mark = [&](int k) {
             if (PROF) { const long long t = clock64(); pf[k] += t - pt; pt = t; }
         };
         pt = pstart;
-        F3Item it;
+        FwdItem it;
         for (int r = 0; r < n_rounds; r++) {
-            if (!f3_item(p, r, it)) continue;
+            if (!fwd_item(p, r, it)) continue;
             const int n = g ? it.n[1] : it.n[0];
             const int q0 = g ? it.q0[1] : it.q0[0], row = q0 + row_t;
             float m_ref = -INFINITY, l_i = 0.f;
             for (int j = 0; j < it.nt; j++) {
                 if (j >= n) {            // the other group's extra tile: keep the token moving
-                    if (PINGPONG) {
-                        asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");
-                        asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");
-                    }
+                    asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");
+                    asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");
                     continue;
                 }
                 const int k0 = j * BK;
@@ -700,7 +274,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
                 }
                 const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
                 // ---- reference maximum; P buffer and O are free / stable once P.V of the previous tile has retired
-                const bool need = (mx - m_ref) * sl2 > F3_RESCALE_LOG2;       // true on the first tile (m_ref = -inf)
+                const bool need = (mx - m_ref) * sl2 > RESCALE_LOG2;       // true on the first tile (m_ref = -inf)
                 mark(1);
                 if (j > 0) {
                     mbar_wait(&pv_done[g], (tg - 1) & 1);
@@ -726,7 +300,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
                 const float msc = m_ref * sl2;
                 // ---- pass 2: probabilities -> bf16 -> swizzled P tile in shared memory
                 mark(2);
-                if (PINGPONG) asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");
+                asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");
                 mark(3);
                 float rs4[4] = {0.f, 0.f, 0.f, 0.f};
                 tmem_ld32(tS, rr[0]);
@@ -768,7 +342,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
                         if (lane == 0) mbar_arrive(&s_empty[g]);
                     }
                 }
-                if (PINGPONG) asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");
+                asm volatile("bar.arrive %0, 64;" ::"r"(bar_other) : "memory");
                 mark(4);
                 l_i += (rs4[0] + rs4[1]) + (rs4[2] + rs4[3]);
                 tc_fence_before();
@@ -803,7 +377,7 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
             // the next item's first P.V (accumulate = 0) overwrites O only after this thread's p_full arrival: ordered
             tc_fence_before();
         }
-        if (PINGPONG && g == 0) asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");    // consume the last token
+        if (g == 0) asm volatile("bar.sync %0, 64;" ::"r"(bar_mine) : "memory");    // consume the last token
         if (PROF && lane == 0 && p.dbg) {
             mark(6);                                   // [6] = epilogues + item bookkeeping + dummy token passes
             for (int k = 0; k < 7; k++) atomicAdd((unsigned long long*)&p.dbg[g * 16 + k], (unsigned long long)pf[k]);
@@ -820,334 +394,6 @@ attn_fwd_tc05_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// forward, fourth generation: the v3 skeleton (persistent CTAs, two query tiles per CTA, O accumulated in TMEM with a lazy
-// rescale, one MMA-issuing warp per group) with TWO threads per query row: 16 softmax warps, four per SM sub-partition.
-// A single warp cannot keep the MUFU pipe busy through the softmax instruction mix (tools/micro/mufu_bench.cu: 13.4 cycles per
-// warp-exponential with one warp per sub-partition, 9.5 with four; the pipe's floor is 8), and with only two warps per
-// sub-partition every barrier wait of one warp idles half of the issue slots.  A thread owns 64 of the 128 keys of a row; the
-// two halves of a row agree on the exact row maximum through 4 bytes of shared memory and a 64-thread named barrier per tile
-// (the two warps involved sit on the same sub-partition), write their own 64-key atom of the P tile, rescale / emit their own
-// 32 output columns and meet once more per item for the row sum.
-//   warp 0: TMA producer   warps 1, 2: MMA issuers of group 0 / 1   warp 3: TMEM allocator
-//   warps 4..19: softmax; warp w -> row quarter w & 3, group (w - 4) >> 3, key half ((w - 4) >> 2) & 1
-// ---------------------------------------------------------------------------------------------
-constexpr int F4_THREADS = 640;
-constexpr int F4_KVS = 3;                                 // K/V stages (one fewer than v3: the exchange area needs 4 KB)
-constexpr int F4_BAR = F3_KV + F4_KVS * 32768;
-constexpr int F4_MX = F4_BAR + 256;                       // float [2 groups][2 slots][2 halves][128 rows]: row-maximum exchange
-constexpr int F4_SMEM = F4_MX + 4096;
-static_assert(F4_SMEM <= 232448 && F3_SMEM <= 232448, "dynamic shared memory of the forward kernels exceeds 227 KB");
-
-template <bool PROF>
-__global__ void __launch_bounds__(F4_THREADS, 1)
-attn_fwd_tc05_v4_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                        const __grid_constant__ CUtensorMap tmV, const FwdParams p) {
-    B200_PDL_TRIGGER();
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + F4_BAR);
-    uint64_t* kv_full = bars + 0;      // [F4_KVS]
-    uint64_t* kv_empty = bars + 4;     // [F4_KVS]  one arrival per MMA warp
-    uint64_t* q_full = bars + 8;       // [2]
-    uint64_t* q_empty = bars + 10;     // [2]
-    uint64_t* s_full = bars + 12;      // [2]
-    uint64_t* s_empty = bars + 14;     // [2]  8 softmax warps
-    uint64_t* p_full = bars + 16;      // [2]  8 softmax warps
-    uint64_t* pv_done = bars + 18;     // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 20);
-    float* mx_s = reinterpret_cast<float*>(smem + F4_MX);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_rounds = (int)(((long long)((p.Sq + BQ - 1) / BQ + 1) / 2 * p.batch * p.n_heads + gridDim.x - 1) / gridDim.x);
-
-    if (warp == 0 && lane == 0) {
-        prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV);
-        for (int s = 0; s < F4_KVS; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 2); }
-        for (int g = 0; g < 2; g++) {
-            mbar_init(&q_full[g], 1); mbar_init(&q_empty[g], 1); mbar_init(&s_full[g], 1); mbar_init(&s_empty[g], 8);
-            mbar_init(&p_full[g], 8); mbar_init(&pv_done[g], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 3) tmem_alloc(tmem_slot, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    // register budget: 640 threads start with 96 registers each (a pool of 61 440 for the CTA); the four housekeeping warps drop
-    // to 56 so that the sixteen softmax warps can take 104 (16 x 32 x 104 + 4 x 32 x 56 = 60 416 <= 61 440 -- a larger request
-    // than the CTA's own pool never succeeds) and hold both 32-column chunks of their half tile across the two passes
-    if (warp < 4) {
-      asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
-      if (warp == 0) {
-        if (lane == 0) {
-            uint32_t T = 0, cq0 = 0, cq1 = 0;
-            F3Item it;
-            for (int r = 0; r < n_rounds; r++) {
-                if (!f3_item(p, r, it)) continue;
-                if (it.n[0] > 0) {
-                    mbar_wait(&q_empty[0], (cq0 & 1) ^ 1);
-                    mbar_expect_tx(&q_full[0], BQ * D * 2);
-                    tma_load_3d(smem + F3_Q, &tmQ, &q_full[0], p.q_col0 + it.h * D, it.q0[0], it.b);
-                    cq0++;
-                }
-                if (it.n[1] > 0) {
-                    mbar_wait(&q_empty[1], (cq1 & 1) ^ 1);
-                    mbar_expect_tx(&q_full[1], BQ * D * 2);
-                    tma_load_3d(smem + F3_Q + 16384, &tmQ, &q_full[1], p.q_col0 + it.h * D, it.q0[1], it.b);
-                    cq1++;
-                }
-                for (int j = 0; j < it.nt; j++, T++) {
-                    const int st = T % F4_KVS;
-                    mbar_wait(&kv_empty[st], ((T / F4_KVS) & 1) ^ 1);
-                    uint8_t* sK = smem + F3_KV + st * 32768;
-                    mbar_expect_tx(&kv_full[st], 2 * BK * D * 2);
-                    tma_load_3d(sK, &tmK, &kv_full[st], p.k_col0 + it.h * D, j * BK, it.b);
-                    tma_load_3d(sK + 16384, &tmV, &kv_full[st], p.v_col0 + it.h * D, j * BK, it.b);
-                }
-            }
-        }
-      } else if (warp == 1 || warp == 2) {
-        if (lane == 0) {
-            const int g = warp - 1;
-            constexpr uint32_t idesc_s = make_idesc(BQ, BK, false, false);    // S[128 x 128] = Q . K^T
-            constexpr uint32_t idesc_pv = make_idesc(BQ, D, false, true);     // O[128 x 64] += P . V (V is [keys, d]: MN-major B)
-            const uint32_t tS = tmem_base + g * 128, tO = tmem_base + 256 + g * 64;
-            const uint64_t dQ0 = make_smem_desc(smem_u32(smem + F3_Q + g * 16384), 16, 1024);
-            const uint64_t dP0 = make_smem_desc(smem_u32(smem + F3_P + g * 32768), 16, 1024);
-            uint32_t T = 0, tg = 0, cq = 0;
-            auto issue_s = [&](uint32_t Tj) {               // S = Q . K_j^T of the K/V tile with running index Tj
-                const int st = Tj % F4_KVS;
-                mbar_wait(&kv_full[st], (Tj / F4_KVS) & 1);
-                const uint64_t dK0 = make_smem_desc(smem_u32(smem + F3_KV + st * 32768), 16, 1024);
-                tc_fence_after();
-#pragma unroll
-                for (int k = 0; k < D / 16; k++) umma_f16(tS, desc_adv(dQ0, k * 32), desc_adv(dK0, k * 32), idesc_s, k > 0);
-                umma_commit(&s_full[g]);
-            };
-            F3Item it;
-            for (int r = 0; r < n_rounds; r++) {
-                if (!f3_item(p, r, it)) continue;
-                const int n = g ? it.n[1] : it.n[0];
-                if (n > 0) { mbar_wait(&q_full[g], cq & 1); cq++; }
-                for (int j = 0; j < it.nt; j++, T++) {
-                    const int st = T % F4_KVS;
-                    if (j < n) {
-                        if (j == 0) {
-                            if (tg > 0) mbar_wait(&s_empty[g], (tg - 1) & 1);      // last tile of the previous item read out
-                            issue_s(T);
-                            if (n == 1) umma_commit(&q_empty[g]);
-                        }
-                        if (j + 1 < n) {                                           // S_{j+1} first: the group never waits for it
-                            mbar_wait(&s_empty[g], tg & 1);
-                            issue_s(T + 1);
-                            if (j + 2 == n) umma_commit(&q_empty[g]);
-                        }
-                        mbar_wait(&p_full[g], tg & 1);
-                        tc_fence_after();
-                        const uint64_t dV0 = make_smem_desc(smem_u32(smem + F3_KV + st * 32768 + 16384), 16384, 1024);
-#pragma unroll
-                        for (int kk = 0; kk < BK / 16; kk++)
-                            umma_f16(tO, desc_adv(dP0, (kk >> 2) * 16384 + (kk & 3) * 32), desc_adv(dV0, kk * 2048), idesc_pv,
-                                     (j > 0 || kk > 0) ? 1u : 0u);
-                        umma_commit(&pv_done[g]);
-                        umma_commit(&kv_empty[st]);
-                        tg++;
-                    } else {
-                        mbar_wait(&kv_full[st], (T / F4_KVS) & 1);                 // the other group's tile: just pass the stage on
-                        mbar_arrive(&kv_empty[st]);
-                    }
-                }
-            }
-        }
-      }
-    } else {
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 104;");
-        const int g = (warp - 4) >> 3;
-        const int half = ((warp - 4) >> 2) & 1;           // keys half*64 .. +63 of every tile, output columns half*32 .. +31
-        const int quarter = warp & 3;
-        const int row_t = quarter * 32 + lane;            // row inside the tile == TMEM lane
-        const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        const uint32_t tS = tmem_base + g * 128 + half * 64 + lane_addr, tO = tmem_base + 256 + g * 64 + half * 32 + lane_addr;
-        const float sl2 = p.scale * LOG2E;
-        const int off = p.Sk - p.Sq;
-        uint8_t* sP = smem + F3_P + g * 32768 + half * 16384 + row_t * 128;      // this thread's 128-byte row of its 64-key atom
-        float* mxg = mx_s + g * 512;                      // [slot][half][row]
-        const int pair_bar = 1 + g * 4 + quarter;         // named barrier of the two warps that share this row quarter
-        uint32_t tg = 0;
-        long long pf[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pt = 0;      // PROF: cycles per phase (lane 0)
-        const long long pstart = PROF ? clock64() : 0;
-        auto mark = [&](int k) {
-            if (PROF) { const long long t = clock64(); pf[k] += t - pt; pt = t; }
-        };
-        pt = pstart;
-        F3Item it;
-        for (int r = 0; r < n_rounds; r++) {
-            if (!f3_item(p, r, it)) continue;
-            const int n = g ? it.n[1] : it.n[0];
-            if (n == 0) continue;
-            const int q0 = g ? it.q0[1] : it.q0[0], row = q0 + row_t;
-            float m_ref = -INFINITY, l_i = 0.f;
-            for (int j = 0; j < n; j++, tg++) {
-                const int k0 = j * BK + half * 64;
-                const bool need_mask = (j * BK + BK - 1 > q0 + off) || (j * BK + BK > p.Sk);
-                const int lim0 = min(row + off, p.Sk - 1) - k0;     // last visible column of this row in this thread's half tile
-                mark(6);
-                mbar_wait(&s_full[g], tg & 1);
-                tc_fence_after();
-                mark(0);
-                uint32_t rr[2][32];
-                // ---- pass 1: row maximum over this thread's 64 keys, then the exact row maximum with the other half
-                float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-                tmem_ld32(tS, rr[0]);
-                tmem_ld32(tS + 32, rr[1]);
-                tmem_ld_wait();
-#pragma unroll
-                for (int c = 0; c < 2; c++) {
-                    if (need_mask) {
-                        const int lim = lim0 - c * 32;
-#pragma unroll
-                        for (int i = 0; i < 32; i++)
-                            mx4[i & 3] = fmaxf(mx4[i & 3], (i > lim) ? -INFINITY : __uint_as_float(rr[c][i]));
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 32; i++) mx4[i & 3] = fmaxf(mx4[i & 3], __uint_as_float(rr[c][i]));
-                    }
-                }
-                float* mslot = mxg + (tg & 1) * 256;
-                mslot[half * 128 + row_t] = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-                asm volatile("bar.sync %0, 64;" ::"r"(pair_bar) : "memory");
-                const float mx = fmaxf(mslot[row_t], mslot[128 + row_t]);
-                // ---- reference maximum; P buffer and O are free / stable once P.V of the previous tile has retired
-                const bool need = (mx - m_ref) * sl2 > F3_RESCALE_LOG2;       // true on the first tile (m_ref = -inf)
-                mark(1);
-                if (j > 0) {
-                    mbar_wait(&pv_done[g], (tg - 1) & 1);
-                    tc_fence_after();
-                }
-                if (__any_sync(0xffffffffu, need)) {
-                    const float m_new = need ? mx : m_ref;
-                    if (j > 0) {
-                        const float alpha = need ? exp2f((m_ref - m_new) * sl2) : 1.f;
-                        uint32_t ro[32];
-                        tmem_ld32(tO, ro);
-                        tmem_ld_wait();
-#pragma unroll
-                        for (int i = 0; i < 32; i++) ro[i] = __float_as_uint(__uint_as_float(ro[i]) * alpha);
-                        tmem_st32(tO, ro);
-                        tmem_st_wait();
-                        l_i *= alpha;
-                    }
-                    m_ref = m_new;
-                }
-                const float msc = m_ref * sl2;
-                mark(2);
-                // ---- pass 2: probabilities -> bf16 -> this half's 64-key atom of the swizzled P tile (S is still in registers)
-                float rs4[4] = {0.f, 0.f, 0.f, 0.f};
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&s_empty[g]);      // both chunks are in registers: the tensor pipe may overwrite S
-#pragma unroll
-                for (int c = 0; c < 2; c++) {
-                    uint32_t pk[16];
-                    if (need_mask) {
-                        const int lim = lim0 - c * 32;
-#pragma unroll
-                        for (int i = 0; i < 32; i += 2) {
-                            const float p0 = (i > lim) ? 0.f : ex2_approx(fmaf(__uint_as_float(rr[c][i]), sl2, -msc));
-                            const float p1 = (i + 1 > lim) ? 0.f : ex2_approx(fmaf(__uint_as_float(rr[c][i + 1]), sl2, -msc));
-                            rs4[(i >> 1) & 3] += p0 + p1;
-                            pk[i >> 1] = pack2(p0, p1);
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 32; i += 2) {
-                            const float p0 = ex2_approx(fmaf(__uint_as_float(rr[c][i]), sl2, -msc));
-                            const float p1 = ex2_approx(fmaf(__uint_as_float(rr[c][i + 1]), sl2, -msc));
-                            rs4[(i >> 1) & 3] += p0 + p1;
-                            pk[i >> 1] = pack2(p0, p1);
-                        }
-                    }
-#pragma unroll
-                    for (int v = 0; v < 4; v++) {
-                        const int chunk = c * 4 + v;
-                        *reinterpret_cast<uint4*>(sP + ((chunk ^ (row_t & 7)) << 4)) =
-                            make_uint4(pk[4 * v], pk[4 * v + 1], pk[4 * v + 2], pk[4 * v + 3]);
-                    }
-                }
-                mark(4);
-                l_i += (rs4[0] + rs4[1]) + (rs4[2] + rs4[3]);
-                tc_fence_before();
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&p_full[g]);
-                mark(5);
-            }
-            // ---- epilogue of the item: the two halves of a row add their sums, then O / l -> bf16 (32 columns per thread)
-            float* lslot = mxg + (tg & 1) * 256;          // the slot the last tile did not use
-            lslot[half * 128 + row_t] = l_i;
-            asm volatile("bar.sync %0, 64;" ::"r"(pair_bar) : "memory");
-            const float l_row = lslot[row_t] + lslot[128 + row_t];
-            mbar_wait(&pv_done[g], (tg - 1) & 1);
-            tc_fence_after();
-            const float inv = l_row > 0.f ? 1.f / l_row : 0.f;
-            bf16* dst = p.o + it.b * p.o_b + (long long)row * p.o_r + it.h * D + half * 32;
-            {
-                uint32_t ro[32];
-                tmem_ld32(tO, ro);
-                tmem_ld_wait();
-                if (row < p.Sq) {
-#pragma unroll
-                    for (int v = 0; v < 4; v++) {
-                        float f[8];
-#pragma unroll
-                        for (int i = 0; i < 8; i++) f[i] = __uint_as_float(ro[v * 8 + i]) * inv;
-                        *reinterpret_cast<uint4*>(dst + v * 8) = pack8(f);
-                    }
-                }
-            }
-            if (p.lse && half == 0 && row < p.Sq)
-                p.lse[((long long)it.b * p.n_heads + it.h) * p.Sq + row] = m_ref * p.scale + logf(l_row);
-            // the next item's first P.V (accumulate = 0) overwrites O only after this thread's p_full arrival: ordered;
-            // its first maximum goes to the other slot, and the pair barrier of that tile orders the reuse of this one
-            tc_fence_before();
-        }
-        if (PROF && lane == 0 && p.dbg) {
-            mark(6);
-            for (int k = 0; k < 7; k++) atomicAdd((unsigned long long*)&p.dbg[g * 16 + k], (unsigned long long)pf[k]);
-            atomicAdd((unsigned long long*)&p.dbg[g * 16 + 7], (unsigned long long)(clock64() - pstart));
-            atomicAdd((unsigned long long*)&p.dbg[g * 16 + 8], (unsigned long long)tg);
-            atomicAdd((unsigned long long*)&p.dbg[g * 16 + 9], 1ull);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 3) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
-}
-
-static int f3_launch(bool pingpong, bool prof, int grid, cudaStream_t stream, const CUtensorMap& tmQ, const CUtensorMap& tmK,
-                     const CUtensorMap& tmV, const FwdParams& p) {
-    static bool init = false;
-    if (!init) {
-        int bad = 0;
-        bad |= cudaFuncSetAttribute(attn_fwd_tc05_v3_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, F3_SMEM) != cudaSuccess;
-        bad |= cudaFuncSetAttribute(attn_fwd_tc05_v3_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, F3_SMEM) != cudaSuccess;
-        bad |= cudaFuncSetAttribute(attn_fwd_tc05_v3_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, F3_SMEM) != cudaSuccess;
-        bad |= cudaFuncSetAttribute(attn_fwd_tc05_v3_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, F3_SMEM) != cudaSuccess;
-        B200_CHECK_ARG(!bad, "attn_causal_fwd_tc: cannot set the shared-memory size of the v3 kernel");
-        init = true;
-    }
-    if (prof) {      // phase profile (tools/attn_fwd_profile.py): instrumented instantiation
-        if (pingpong) attn_fwd_tc05_v3_kernel<true, true><<<grid, F3_THREADS, F3_SMEM, stream>>>(tmQ, tmK, tmV, p);
-        else attn_fwd_tc05_v3_kernel<false, true><<<grid, F3_THREADS, F3_SMEM, stream>>>(tmQ, tmK, tmV, p);
-    } else if (pingpong) attn_fwd_tc05_v3_kernel<true, false><<<grid, F3_THREADS, F3_SMEM, stream>>>(tmQ, tmK, tmV, p);
-    else attn_fwd_tc05_v3_kernel<false, false><<<grid, F3_THREADS, F3_SMEM, stream>>>(tmQ, tmK, tmV, p);
-    return B200_OK;
-}
 }   // namespace
 
 static long long* g_attn_dbg = nullptr;
@@ -1178,43 +424,19 @@ extern "C" int b200_attn_causal_fwd_tc(const void* q, const void* k, const void*
     p.batch = batch; p.n_heads = n_heads; p.Sq = Sq; p.Sk = Sk; p.H = (int)W;
     p.q_col0 = p.k_col0 = p.v_col0 = 0;
     p.scale = scale;
-    p.dbg = nullptr;
-    static int gen = 0;
-    static bool pingpong = true;
-    if (!gen) {
-        // B200_ATTN_FWD_TC=v1 / v2 select the earlier generations (see the file header)
-        const char* e = getenv("B200_ATTN_FWD_TC");
-        gen = (e && !strcmp(e, "v1")) ? 1 : (e && !strcmp(e, "v2")) ? 2 : (e && !strcmp(e, "v4")) ? 4 : 3;
-        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_v4_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, F4_SMEM), "attn_tc v4 smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_v4_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, F4_SMEM), "attn_tc v4 smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES), "attn_tc smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                       cudaSharedmemCarveoutMaxShared), "attn_tc carveout");
-        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_v2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F2_SMEM), "attn_tc v2 smem");
-        const char* pp = getenv("B200_ATTN_FWD_PINGPONG");
-        pingpong = !(pp && pp[0] == '0');
+    p.dbg = g_attn_dbg;
+    static bool configured = false;
+    if (!configured) {
+        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_FWD_BYTES),
+                  "attn_tc smem");
+        B200_CUDA(cudaFuncSetAttribute(attn_fwd_tc05_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_FWD_BYTES),
+                  "attn_tc smem");
+        configured = true;
     }
-    if (gen == 4) {
-        const long long items = (long long)(((Sq + BQ - 1) / BQ + 1) / 2) * batch * n_heads;
-        const int g4 = (int)(items < b200_num_sms() ? items : b200_num_sms());
-        p.dbg = g_attn_dbg;
-        if (p.dbg) attn_fwd_tc05_v4_kernel<true><<<g4, F4_THREADS, F4_SMEM, stream>>>(tmQ, tmK, tmV, p);
-        else attn_fwd_tc05_v4_kernel<false><<<g4, F4_THREADS, F4_SMEM, stream>>>(tmQ, tmK, tmV, p);
-        B200_CHECK_LAUNCH("attn_causal_fwd_tc");
-        return B200_OK;
-    }
-    if (gen == 3) {
-        const long long items = (long long)(((Sq + BQ - 1) / BQ + 1) / 2) * batch * n_heads;
-        const int g3 = (int)(items < b200_num_sms() ? items : b200_num_sms());
-        p.dbg = g_attn_dbg;
-        const int rc3 = f3_launch(pingpong, p.dbg != nullptr, g3, stream, tmQ, tmK, tmV, p);
-        if (rc3) return rc3;
-        B200_CHECK_LAUNCH("attn_causal_fwd_tc");
-        return B200_OK;
-    }
-    dim3 grid(batch * n_heads, (Sq + BQ - 1) / BQ);   // tiles on the slow index: longest first across all heads
-    if (gen == 2) attn_fwd_tc05_v2_kernel<<<grid, F2_THREADS, F2_SMEM, stream>>>(tmQ, tmK, tmV, p);
-    else attn_fwd_tc05_kernel<<<grid, NTHREADS, SMEM_BYTES, stream>>>(tmQ, tmK, tmV, p);
+    const long long items = (long long)(((Sq + BQ - 1) / BQ + 1) / 2) * batch * n_heads;
+    const int grid = (int)(items < b200_num_sms() ? items : b200_num_sms());
+    if (p.dbg) attn_fwd_tc05_kernel<true><<<grid, FWD_THREADS, SMEM_FWD_BYTES, stream>>>(tmQ, tmK, tmV, p);
+    else attn_fwd_tc05_kernel<false><<<grid, FWD_THREADS, SMEM_FWD_BYTES, stream>>>(tmQ, tmK, tmV, p);
     B200_CHECK_LAUNCH("attn_causal_fwd_tc");
     return B200_OK;
 }
@@ -1244,26 +466,21 @@ constexpr int SB_DQ = SB_DS + 32768;             // fp32 dQ tile for the TMA red
 constexpr int SB_LSE = SB_DQ + 32768;            // float [2][2][128]: lse, delta per stage parity
 constexpr int SB_BAR = SB_LSE + 2048;
 constexpr int SMEM_BWD_BYTES = SB_BAR + 192;
-constexpr int BWD_DEFAULT_UNITS = 2;
-constexpr int BWD_DEFAULT_LDM = 2;
 
+// n_heads / Sq fill the slot between delta and dk: that keeps dv, dk_r, dv_r and rope_sin 16-byte aligned, and ptxas
+// schedules the epilogue's parameter loads by that alignment
 struct BwdParams {
     const float* lse;
     const float* delta;
-    float* dq_acc;               // fp32 [batch, Sq, n_heads*64] accumulator (pre-zeroed)
+    int n_heads, Sq;
     bf16* dk;
     bf16* dv;
     long long dk_b, dk_r, dv_b, dv_r;
-    long long dqa_b, dqa_r;
     const bf16* rope_cos;        // optional fused RoPE backward on dK (dQ gets it in the finalize kernel)
     const bf16* rope_sin;
-    int n_heads, Sq, Sk;
+    int Sk;
     float scale;
 };
-
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
 
 // fp32 tile in shared memory += into global memory through the TMA unit (one instruction per 16 KB box instead of
 // 1024 per-lane red.global instructions)
@@ -1272,30 +489,22 @@ __device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* tm, uint32_
                  ::"l"(tm), "r"(smem_addr), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 
-// DQ_MODE: 0 = dK/dV only (dQ by the separate kernel below), 1 = dQ through red.global.add.v4.f32,
-//          2 = dQ tile staged in shared memory and added with cp.reduce.async.bulk.tensor
-// NU: pipeline units per query tile.  2 = half tiles (64 queries): two math groups of 8 warps.  4 = quarter tiles (32 queries):
-//     four math groups of 4 warps, one warp of every group on each SM sub-partition, i.e. four independent dependent chains
-//     per scheduler instead of two lockstepped pairs (same thread -> element mapping, same TMEM / shared-memory layout; only
-//     the hand-over granularity between the MMA-issuing thread and the math warps changes, and S^T / dP^T become N = 32 UMMAs).
-// LDM: how the math warps get lse / delta of their 32 query columns.  0 = every warp stages them in shared memory itself (the four
-//     quarter-warps that share the columns write identical words; __syncwarp only).  1 = no staging: uniform 16-byte loads from
-//     global memory (L1 hits; the lines are prefetched one iteration ahead).  2 = one writer warp per column group stages the
-//     NEXT iteration's values before its pds_full arrival: the MMA thread issues S^T of that iteration only after all arrivals
-//     and the readers acquire s_full, so the hand-over is ordered by the mbarriers that are there anyway.
-template <int DQ_MODE, int NU, int LDM>
+// lse / delta of a group's 32 query columns reach its math warps through shared memory: one writer warp per column group
+// stages the NEXT iteration's values before its pds_full arrival; the MMA thread issues S^T of that iteration only after all
+// arrivals and the readers acquire s_full, so the hand-over is ordered by the mbarriers that are there anyway.
+// compute-sanitizer's racecheck does not follow an ordering that passes through tcgen05.commit, so it reports these stores
+// against the reads (profiles/r2_sanitizer_attention.txt).
 __global__ void __launch_bounds__(BWD_THREADS, 1)
 attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                      const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
                      const __grid_constant__ CUtensorMap tmDQ, const BwdParams p) {
-    constexpr bool WITH_DQ = DQ_MODE != 0;
     extern __shared__ __align__(1024) uint8_t smem[];
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SB_BAR);
     uint64_t* kv_full = bars + 0;
     uint64_t* q_full = bars + 1;      // [QS]
     uint64_t* q_empty = bars + 5;     // [QS]
-    uint64_t* s_full = bars + 9;      // [NU]  one per pipeline unit of a tile
-    uint64_t* pds_full = bars + 13;   // [NU]
+    uint64_t* s_full = bars + 9;      // [2]  one per pipeline unit (half tile)
+    uint64_t* pds_full = bars + 13;   // [2]
     uint64_t* dq_full = bars + 17;
     uint64_t* dq_empty = bars + 18;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 19);
@@ -1317,12 +526,12 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV); prefetch_tmap(&tmdO);
         mbar_init(kv_full, 1);
         for (int s = 0; s < QS; s++) { mbar_init(&q_full[s], 1); mbar_init(&q_empty[s], 1); }
-        for (int s = 0; s < NU; s++) { mbar_init(&s_full[s], 1); mbar_init(&pds_full[s], BWD_CWARPS / NU); }
+        for (int s = 0; s < 2; s++) { mbar_init(&s_full[s], 1); mbar_init(&pds_full[s], BWD_CWARPS / 2); }
         mbar_init(dq_full, 1); mbar_init(dq_empty, BWD_CWARPS / 2);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) tmem_alloc(tmem_slot, 512);
-    if (LDM == 2 && warp >= 2 && (warp & 3) == 0) {
+    if (warp >= 2 && (warp & 3) == 0) {
         // writer warps (row quarter 0): lse / delta of the first iteration, visible to everyone through the barrier below
         const int cw_ = warp - 2, qc_ = (cw_ >> 3) * 64 + ((cw_ >> 2) & 1) * 32;
         const int qi = i0 * BQ + qc_ + lane;
@@ -1355,7 +564,7 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         }
     } else if (warp == 1) {
         if (lane == 0 && n_it > 0) {
-            constexpr uint32_t id_s = make_idesc(128, 128 / NU, false, false);  // S^T, dP^T of one unit (64 or 32 queries)
+            constexpr uint32_t id_s = make_idesc(128, 64, false, false);      // S^T, dP^T of one unit (64 queries)
             constexpr uint32_t id_kv = make_idesc(128, 64, false, true);      // dV, dK : A K-major (smem P^T/dS^T), B MN-major
             constexpr uint32_t id_dq = make_idesc(128, 64, true, true);       // dQ     : A = dS (MN-major view of dS^T), B = K MN-major
             const uint32_t sK = smem_u32(smem + SB_K), sV = smem_u32(smem + SB_V);
@@ -1368,14 +577,13 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
             // The pipeline unit is a half tile: 64 queries x 128 keys.  Unit u = (tile u/2, half u&1) owns TMEM buffer
             // u&1 and P^T/dS^T atom u&1, so S^T/dP^T of unit u+2 are produced while the math warps work on unit u+1
             // and the tensor pipe never sits on the critical path.
-            const int n_units = NU * n_it;
+            const int n_units = 2 * n_it;
             auto issue_s = [&](int u) {
-                const int it_ = u / NU, g = u % NU, st = it_ % QS;
-                const int hb = (NU == 4) ? (g >> 1) : g, cgi = (NU == 4) ? (g & 1) : 0;
+                const int it_ = u / 2, g = u % 2, st = it_ % QS;
                 if (g == 0) mbar_wait(&q_full[st], (uint32_t)((it_ / QS) & 1));
-                const uint32_t sQ = smem_u32(smem + SB_Q + st * 32768) + hb * 8192 + cgi * 4096;   // 64 / 32 query rows x 128 B
+                const uint32_t sQ = smem_u32(smem + SB_Q + st * 32768) + g * 8192;   // 64 query rows x 128 B
                 const uint64_t dQk = make_smem_desc(sQ, 16, 1024), dOk = make_smem_desc(sQ + 16384, 16, 1024);
-                const uint32_t tS = tSB + hb * 128 + cgi * 32, tdP = tS + 64;
+                const uint32_t tS = tSB + g * 128, tdP = tS + 64;
                 tc_fence_after();
 #pragma unroll
                 for (int k = 0; k < D / 16; k++) umma_f16(tS, desc_adv(dKk, k * 32), desc_adv(dQk, k * 32), id_s, k > 0);
@@ -1384,39 +592,34 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
                 umma_commit(&s_full[g]);
             };
 #pragma unroll
-            for (int u = 0; u < NU; u++)
+            for (int u = 0; u < 2; u++)
                 if (u < n_units) issue_s(u);
             for (int u = 0; u < n_units; u++) {
-                const int it = u / NU, g = u % NU, st_cur = it % QS;
-                const int hb = (NU == 4) ? (g >> 1) : g, cgi = (NU == 4) ? (g & 1) : 0;
+                const int it = u / 2, g = u % 2, st_cur = it % QS;
                 const uint32_t sQ = smem_u32(smem + SB_Q + st_cur * 32768);
                 const uint64_t dQmn = make_smem_desc(sQ, 16384, 1024), dOmn = make_smem_desc(sQ + 16384, 16384, 1024);
                 mbar_wait(&pds_full[g], (uint32_t)(it & 1));    // P^T / dS^T columns of this unit written; its TMEM buffer is free
                 tc_fence_after();
 #pragma unroll
-                for (int k = 0; k < 8 / NU; k++) {
-                    const int k4 = cgi * 2 + k;                // 16 query rows per step inside the half's 64-query atom
-                    const int kk = hb * 4 + k4;
-                    umma_f16(tdV, desc_adv(dPk, hb * 16384 + k4 * 32), desc_adv(dOmn, kk * 2048), id_kv, (u > 0 || k > 0) ? 1u : 0u);
+                for (int k = 0; k < 4; k++) {                  // 16 query rows per step inside the half's 64-query atom
+                    const int kk = g * 4 + k;
+                    umma_f16(tdV, desc_adv(dPk, g * 16384 + k * 32), desc_adv(dOmn, kk * 2048), id_kv, (u > 0 || k > 0) ? 1u : 0u);
                 }
 #pragma unroll
-                for (int k = 0; k < 8 / NU; k++) {
-                    const int k4 = cgi * 2 + k;
-                    const int kk = hb * 4 + k4;
-                    umma_f16(tdK, desc_adv(dDSk, hb * 16384 + k4 * 32), desc_adv(dQmn, kk * 2048), id_kv, (u > 0 || k > 0) ? 1u : 0u);
+                for (int k = 0; k < 4; k++) {
+                    const int kk = g * 4 + k;
+                    umma_f16(tdK, desc_adv(dDSk, g * 16384 + k * 32), desc_adv(dQmn, kk * 2048), id_kv, (u > 0 || k > 0) ? 1u : 0u);
                 }
-                if (g == NU - 1) {
-                    if (WITH_DQ) {
-                        mbar_wait(dq_empty, (uint32_t)((it & 1) ^ 1));      // previous dQ tile drained
-                        tc_fence_after();
+                if (g == 1) {
+                    mbar_wait(dq_empty, (uint32_t)((it & 1) ^ 1));      // previous dQ tile drained
+                    tc_fence_after();
 #pragma unroll
-                        for (int kk = 0; kk < BK / 16; kk++)   // K dimension = keys: 16 key rows per step
-                            umma_f16(tdQ, desc_adv(dDSmn, kk * 2048), desc_adv(dKmn, kk * 2048), id_dq, kk > 0);
-                    }
+                    for (int kk = 0; kk < BK / 16; kk++)   // K dimension = keys: 16 key rows per step
+                        umma_f16(tdQ, desc_adv(dDSmn, kk * 2048), desc_adv(dKmn, kk * 2048), id_dq, kk > 0);
                     umma_commit(dq_full);
                     umma_commit(&q_empty[st_cur]);
                 }
-                if (u + NU < n_units) issue_s(u + NU);         // one tile ahead: not urgent, goes after this unit's dV/dK/dQ
+                if (u + 2 < n_units) issue_s(u + 2);         // one tile ahead: not urgent, goes after this unit's dV/dK/dQ
             }
         }
     } else {
@@ -1425,8 +628,7 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         // + fence) the other is in its exp2/FMA stretch.  thread = (key row, 32 of the 64 query columns).
         const int cw = warp - 2;                       // 0..15
         const int quarter = warp & 3;
-        const int grp = cw >> 3;                       // half tile index hb
-        const int ug = (NU == 4) ? (cw >> 2) : grp;    // pipeline unit == math group of this warp
+        const int hb = cw >> 3;                        // half tile == pipeline unit == math group of this warp
         const int cgi = (cw >> 2) & 1;                 // which 32 query columns of the half tile
         const int gtid = (cw & 7) * 32 + lane;         // 0..255 inside the group
         const int key_t = quarter * 32 + lane;         // key row inside the tile == TMEM lane
@@ -1435,15 +637,12 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         const float sl2 = p.scale * LOG2E;
         const float* lse_g = p.lse + ((long long)b * p.n_heads + h) * p.Sq;
         const float* delta_g = p.delta + ((long long)b * p.n_heads + h) * p.Sq;
-        const int hb = grp;
         const int qc0 = hb * 64 + cgi * 32;            // first query column (inside the tile) of this thread
         uint8_t* sP = smem + SB_P + hb * 16384 + key_t * 128;
         uint8_t* sDS = smem + SB_DS + hb * 16384 + key_t * 128;
-        // lse / delta of this warp's 32 query columns (lane i -> column qc0 + i), fetched one iteration ahead so the global load
-        // latency hides behind the previous iteration.  Every warp stages the values it reads itself (the four quarter-warps
-        // that share the columns write identical words), so a __syncwarp orders the stores against the broadcast loads and
-        // no group-wide barrier sits on the critical path; the slot parity covers the one iteration two warps can be apart
-        // (S_{it+1} of this half tile is issued only after all eight warps arrived on pds_full for it).
+        // lse / delta of this warp's 32 query columns (lane i -> column qc0 + i), fetched one iteration ahead by the writer warp
+        // so the global load latency hides behind the previous iteration; the slot parity covers the one iteration two warps can
+        // be apart (S_{it+1} of this half tile is issued only after all eight warps arrived on pds_full for it).
         auto fetch_ld = [&](int it_, float& lse_v, float& delta_v) {
             const int qi = (i0 + it_) * BQ + qc0 + lane;
             const bool ok = it_ < n_it && qi < p.Sq;
@@ -1458,79 +657,36 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(dq_empty);                  // TMEM tile is free for the next dQ MMAs
-            if (DQ_MODE == 1) {
-                const int qrow = q0_tile + key_t;                   // (lane index means query row here)
-                if (qrow < p.Sq) {
-                    float* dst = p.dq_acc + b * p.dqa_b + (long long)qrow * p.dqa_r + h * D + cgi * 32;
+            // the previous TMA reduce must have finished reading the staging tile before it is overwritten
+            if (gtid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+            asm volatile("bar.sync 1, 256;" ::: "memory");
+            uint8_t* dst = smem + SB_DQ + cgi * 16384 + key_t * 128;
 #pragma unroll
-                    for (int v = 0; v < 8; v++)
-                        red_add_v4(dst + v * 4, __uint_as_float(r[4 * v]), __uint_as_float(r[4 * v + 1]),
-                                   __uint_as_float(r[4 * v + 2]), __uint_as_float(r[4 * v + 3]));
-                }
-            } else {
-                // the previous TMA reduce must have finished reading the staging tile before it is overwritten
-                if (gtid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                asm volatile("bar.sync 1, 256;" ::: "memory");
-                uint8_t* dst = smem + SB_DQ + cgi * 16384 + key_t * 128;
-#pragma unroll
-                for (int v = 0; v < 8; v++)
-                    *reinterpret_cast<uint4*>(dst + ((v ^ (key_t & 7)) << 4)) = make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]);
-                fence_proxy_async_smem();
-                asm volatile("bar.sync 3, 256;" ::: "memory");
-                if (gtid == 0) {
-                    tma_reduce_add_3d(&tmDQ, smem_u32(smem + SB_DQ), h * D, q0_tile, b);
-                    tma_reduce_add_3d(&tmDQ, smem_u32(smem + SB_DQ + 16384), h * D + 32, q0_tile, b);
-                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                }
+            for (int v = 0; v < 8; v++)
+                *reinterpret_cast<uint4*>(dst + ((v ^ (key_t & 7)) << 4)) = make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]);
+            fence_proxy_async_smem();
+            asm volatile("bar.sync 3, 256;" ::: "memory");
+            if (gtid == 0) {
+                tma_reduce_add_3d(&tmDQ, smem_u32(smem + SB_DQ), h * D, q0_tile, b);
+                tma_reduce_add_3d(&tmDQ, smem_u32(smem + SB_DQ + 16384), h * D + 32, q0_tile, b);
+                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
         };
-        const bool drainer = WITH_DQ && grp == 0;
+        const bool drainer = hb == 0;
         float lse_next = 0.f, delta_next = 0.f;
-        const bool writer = (LDM == 2) && quarter == 0;
-        if (LDM == 0) fetch_ld(0, lse_next, delta_next);
+        const bool writer = quarter == 0;
         for (int it = 0; it < n_it; it++) {
             const int q0 = (i0 + it) * BQ;
-            if (LDM == 0) {
-                lse_s[(it & 1) * 128 + qc0 + lane] = lse_next;
-                delta_s[(it & 1) * 128 + qc0 + lane] = delta_next;
-                fetch_ld(it + 1, lse_next, delta_next);
-                __syncwarp();
-            } else if (LDM == 2) {
-                if (writer) fetch_ld(it + 1, lse_next, delta_next);     // stored before this iteration's pds_full arrival
-            } else if (lane < 2 && it + 1 < n_it) {
-                // pull the next iteration's line of lse (lane 0) / delta (lane 1) into L1
-                const int qn = (i0 + it + 1) * BQ + qc0;
-                if (qn < p.Sq) asm volatile("prefetch.global.L1 [%0];" ::"l"((lane ? delta_g : lse_g) + qn));
-            }
+            if (writer) fetch_ld(it + 1, lse_next, delta_next);     // stored before this iteration's pds_full arrival
             const bool need_mask = (k0 + BK - 1 > q0 + off) || (k0 + BK > p.Sk) || (q0 + BQ > p.Sq);
             const float* lse_t = lse_s + (it & 1) * 128 + qc0;
             const float* delta_t = delta_s + (it & 1) * 128 + qc0;
-            mbar_wait(&s_full[ug], (uint32_t)(it & 1));
+            mbar_wait(&s_full[hb], (uint32_t)(it & 1));
             tc_fence_after();
             uint32_t pk[16], dk_[16];
 #pragma unroll
             for (int hc = 0; hc < 2; hc++) {               // two chunks of 16 columns keep the register footprint flat
                 uint32_t rs[16], rd[16];
-                float lse_r[16], delta_r[16];              // LDM == 1: this chunk's values straight from global memory
-                if (LDM == 1) {
-                    const int qb = q0 + qc0 + hc * 16;
-                    if (qb + 16 <= p.Sq) {
-#pragma unroll
-                        for (int v = 0; v < 4; v++) {
-                            const float4 a4 = __ldg(reinterpret_cast<const float4*>(lse_g + qb) + v);
-                            const float4 d4 = __ldg(reinterpret_cast<const float4*>(delta_g + qb) + v);
-                            lse_r[4 * v] = a4.x * LOG2E; lse_r[4 * v + 1] = a4.y * LOG2E; lse_r[4 * v + 2] = a4.z * LOG2E; lse_r[4 * v + 3] = a4.w * LOG2E;
-                            delta_r[4 * v] = d4.x; delta_r[4 * v + 1] = d4.y; delta_r[4 * v + 2] = d4.z; delta_r[4 * v + 3] = d4.w;
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 16; i++) {
-                            const bool ok = qb + i < p.Sq;
-                            lse_r[i] = ok ? __ldg(lse_g + qb + i) * LOG2E : 0.f;
-                            delta_r[i] = ok ? __ldg(delta_g + qb + i) : 0.f;
-                        }
-                    }
-                }
                 tmem_ld16(tSB + hb * 128 + lane_addr + cgi * 32 + hc * 16, rs);
                 tmem_ld16(tSB + hb * 128 + 64 + lane_addr + cgi * 32 + hc * 16, rd);
                 tmem_ld_wait();
@@ -1544,10 +700,10 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
 #pragma unroll
                         for (int e = 0; e < 2; e++) {
                             const int qq = hc * 16 + i + e;
-                            float pr = ex2_approx(fmaf(__uint_as_float(rs[i + e]), sl2, -(LDM == 1 ? lse_r[i + e] : lse_t[qq])));
+                            float pr = ex2_approx(fmaf(__uint_as_float(rs[i + e]), sl2, -lse_t[qq]));
                             if (qq < lo || qq >= hi) pr = 0.f;
                             pv[e] = pr;
-                            dsv[e] = pr * (__uint_as_float(rd[i + e]) - (LDM == 1 ? delta_r[i + e] : delta_t[qq]));
+                            dsv[e] = pr * (__uint_as_float(rd[i + e]) - delta_t[qq]);
                         }
                         pk[hc * 8 + (i >> 1)] = pack2(pv[0], pv[1]);
                         dk_[hc * 8 + (i >> 1)] = pack2(dsv[0], dsv[1]);
@@ -1560,9 +716,9 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
 #pragma unroll
                         for (int e = 0; e < 2; e++) {
                             const int qq = hc * 16 + i + e;
-                            const float pr = ex2_approx(fmaf(__uint_as_float(rs[i + e]), sl2, -(LDM == 1 ? lse_r[i + e] : lse_t[qq])));
+                            const float pr = ex2_approx(fmaf(__uint_as_float(rs[i + e]), sl2, -lse_t[qq]));
                             pv[e] = pr;
-                            dsv[e] = pr * (__uint_as_float(rd[i + e]) - (LDM == 1 ? delta_r[i + e] : delta_t[qq]));
+                            dsv[e] = pr * (__uint_as_float(rd[i + e]) - delta_t[qq]);
                         }
                         pk[hc * 8 + (i >> 1)] = pack2(pv[0], pv[1]);
                         dk_[hc * 8 + (i >> 1)] = pack2(dsv[0], dsv[1]);
@@ -1587,7 +743,7 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
             tc_fence_before();
             fence_proxy_async_smem();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&pds_full[ug]);
+            if (lane == 0) mbar_arrive(&pds_full[hb]);
             if (drainer && it > 0) drain_dq(q0 - BQ);   // off the critical path
         }
         if (n_it > 0) {
@@ -1595,7 +751,7 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
             tc_fence_after();
             if (drainer) {
                 drain_dq((i0 + n_it - 1) * BQ);
-                if (DQ_MODE == 2 && gtid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+                if (gtid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
             }
         }
         // epilogue: warps 2..9 write dK (two 16-column groups that form RoPE pairs d, d+32), warps 10..17 write dV
@@ -1658,225 +814,6 @@ attn_bwd_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// dQ kernel (no atomics): one CTA = 128 query rows of one (batch, head), looping over the key tiles up to the
-// diagonal.  S = Q.K_j^T and dP = dO.V_j^T are recomputed on the tensor cores (cheap: the tensor pipe is mostly idle
-// in the backward pass, while a red.global-based accumulation of dQ saturates the L2 atomic units -- measured),
-// dS = P o (dP - delta) is written row-wise to swizzled shared memory and dQ += dS . K_j accumulates in TMEM.
-// ---------------------------------------------------------------------------------------------
-constexpr int SQ_Q = 0, SQ_DO = 16384;
-constexpr int KVS = 4;                           // (K, V) stages
-constexpr int SQ_KV = 32768;                     // KVS stages x (K 16 KB + V 16 KB)
-constexpr int SQ_DS = SQ_KV + KVS * 32768;       // dS [128 q x 128 keys]: two 64-key atoms
-constexpr int SQ_BAR = SQ_DS + 32768;
-constexpr int SMEM_DQ_BYTES = SQ_BAR + 128;
-
-struct DqParams {
-    const float* lse;
-    const float* delta;
-    bf16* dq;
-    long long dq_b, dq_r;
-    const bf16* rope_cos;
-    const bf16* rope_sin;
-    int n_heads, Sq, Sk;
-    float scale;
-    long long* dbg;              // optional clock64 trace of CTA (0,0) (bring-up / tuning only)
-};
-
-__global__ void __launch_bounds__(BWD_THREADS, 1)
-attn_bwd_dq_tc05_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                        const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO, const DqParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SQ_BAR);
-    uint64_t* q_full = bars + 0;
-    uint64_t* kv_full = bars + 1;     // [KVS]
-    uint64_t* kv_empty = bars + 5;    // [KVS]
-    uint64_t* s_full = bars + 9;
-    uint64_t* ds_full = bars + 10;
-    uint64_t* dq_done = bars + 11;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 12);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int qt = gridDim.y - 1 - blockIdx.y;       // long tiles first
-    const int bh = blockIdx.x;
-    const int b = bh / p.n_heads, h = bh % p.n_heads;
-    const int q0 = qt * BQ;
-    const int off = p.Sk - p.Sq;
-    int n_kv = min((p.Sk + BK - 1) / BK, (q0 + BQ - 1 + off) / BK + 1);
-    if (n_kv < 1) n_kv = 1;
-    const bool trace = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0;
-#define TRACE(slot, jj) do { if (trace && (jj) < 16) p.dbg[(jj) * 8 + (slot)] = clock64(); } while (0)
-
-    if (warp == 0 && lane == 0) {
-        prefetch_tmap(&tmQ); prefetch_tmap(&tmK); prefetch_tmap(&tmV); prefetch_tmap(&tmdO);
-        mbar_init(q_full, 1);
-        for (int s = 0; s < KVS; s++) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 1); }
-        mbar_init(s_full, 1); mbar_init(ds_full, BWD_CWARPS); mbar_init(dq_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(tmem_slot, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tS = tmem_base, tdP = tmem_base + 128, tdQ = tmem_base + 256;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_expect_tx(q_full, 2 * BQ * D * 2);
-            tma_load_3d(smem + SQ_Q, &tmQ, q_full, h * D, q0, b);
-            tma_load_3d(smem + SQ_DO, &tmdO, q_full, h * D, q0, b);
-            int stage = 0; uint32_t phase = 0;
-            for (int j = 0; j < n_kv; j++) {
-                mbar_wait(&kv_empty[stage], phase ^ 1);
-                uint8_t* sK = smem + SQ_KV + stage * 32768;
-                mbar_expect_tx(&kv_full[stage], 2 * BK * D * 2);
-                tma_load_3d(sK, &tmK, &kv_full[stage], h * D, j * BK, b);
-                tma_load_3d(sK + 16384, &tmV, &kv_full[stage], h * D, j * BK, b);
-                if (++stage == KVS) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            constexpr uint32_t id_s = make_idesc(128, 128, false, false);
-            constexpr uint32_t id_dq = make_idesc(128, 64, false, true);      // A = dS (K-major over keys), B = K MN-major
-            const uint32_t sQ = smem_u32(smem + SQ_Q), sdO = smem_u32(smem + SQ_DO), sDS = smem_u32(smem + SQ_DS);
-            mbar_wait(q_full, 0);
-            int stage = 0; uint32_t kv_phase = 0, ph = 0;
-            const uint64_t dQk = make_smem_desc(sQ, 16, 1024), dOk = make_smem_desc(sdO, 16, 1024);
-            const uint64_t dDSk = make_smem_desc(sDS, 16, 1024);
-            auto issue_s = [&](int st) {
-                const uint32_t sK = smem_u32(smem + SQ_KV + st * 32768);
-                const uint64_t dKk = make_smem_desc(sK, 16, 1024), dVk = make_smem_desc(sK + 16384, 16, 1024);
-                tc_fence_after();
-#pragma unroll
-                for (int k = 0; k < D / 16; k++) umma_f16(tS, desc_adv(dQk, k * 32), desc_adv(dKk, k * 32), id_s, k > 0);
-#pragma unroll
-                for (int k = 0; k < D / 16; k++) umma_f16(tdP, desc_adv(dOk, k * 32), desc_adv(dVk, k * 32), id_s, k > 0);
-                umma_commit(s_full);
-            };
-            mbar_wait(&kv_full[0], 0);
-            TRACE(0, 0);
-            issue_s(0);
-            for (int j = 0; j < n_kv; j++) {
-                const uint64_t dKmn = make_smem_desc(smem_u32(smem + SQ_KV + stage * 32768), 16384, 1024);
-                mbar_wait(ds_full, ph);           // dS_j in shared memory; S / dP TMEM free again
-                TRACE(1, j);
-                tc_fence_after();
-#pragma unroll
-                for (int kk = 0; kk < BK / 16; kk++)
-                    umma_f16(tdQ, desc_adv(dDSk, (kk >> 2) * 16384 + (kk & 3) * 32), desc_adv(dKmn, kk * 2048), id_dq,
-                             (j > 0 || kk > 0) ? 1u : 0u);
-                umma_commit(&kv_empty[stage]);
-                if (++stage == KVS) { stage = 0; kv_phase ^= 1; }
-                if (j + 1 < n_kv) {
-                    mbar_wait(&kv_full[stage], kv_phase);
-                    TRACE(2, j);
-                    issue_s(stage);               // in order behind the dQ MMAs: they have finished reading dS_j by then
-                    TRACE(0, j + 1);
-                } else {
-                    umma_commit(dq_done);
-                }
-                ph ^= 1;
-            }
-        }
-    } else {
-        const int cw = warp - 2;
-        const int quarter = warp & 3;
-        const int cg = cw >> 2;                        // 32 of the 128 key columns
-        const int row_t = quarter * 32 + lane;
-        const int row = q0 + row_t;
-        const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-        const float sl2 = p.scale * LOG2E;
-        const long long sidx = ((long long)b * p.n_heads + h) * p.Sq + row;
-        const float lse_r = row < p.Sq ? p.lse[sidx] * LOG2E : 0.f;
-        const float delta_r = row < p.Sq ? p.delta[sidx] : 0.f;
-        uint8_t* sDS = smem + SQ_DS + (cg >> 1) * 16384 + row_t * 128;
-        uint32_t ph = 0;
-        for (int j = 0; j < n_kv; j++) {
-            const int k0 = j * BK;
-            const bool need_mask = (k0 + BK - 1 > q0 + off) || (k0 + BK > p.Sk) || (q0 + BQ > p.Sq);
-            mbar_wait(s_full, ph);
-            if (warp == 2 && lane == 0) TRACE(3, j);
-            tc_fence_after();
-            uint32_t rs[32], rd[32];
-            tmem_ld32(tS + lane_addr + cg * 32, rs);
-            tmem_ld32(tdP + lane_addr + cg * 32, rd);
-            tmem_ld_wait();
-            if (warp == 2 && lane == 0) TRACE(4, j);
-            uint32_t pk[16];
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-                float dsv[2];
-#pragma unroll
-                for (int e = 0; e < 2; e++) {
-                    float pr = ex2_approx(fmaf(__uint_as_float(rs[i + e]), sl2, -lse_r));
-                    if (need_mask) {
-                        const int key = k0 + cg * 32 + i + e;
-                        if (key > row + off || key >= p.Sk || row >= p.Sq) pr = 0.f;
-                    }
-                    dsv[e] = pr * (__uint_as_float(rd[i + e]) - delta_r);
-                }
-                pk[i >> 1] = pack2(dsv[0], dsv[1]);
-            }
-#pragma unroll
-            for (int v = 0; v < 4; v++) {
-                const int chunk = (cg & 1) * 4 + v;
-                *reinterpret_cast<uint4*>(sDS + ((chunk ^ (row_t & 7)) << 4)) =
-                    make_uint4(pk[4 * v], pk[4 * v + 1], pk[4 * v + 2], pk[4 * v + 3]);
-            }
-            if (warp == 2 && lane == 0) TRACE(5, j);
-            tc_fence_before();
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(ds_full);
-            if (warp == 2 && lane == 0) TRACE(6, j);
-            ph ^= 1;
-        }
-        // epilogue: dQ = scale * tdQ (+ RoPE backward on the (d, d+32) pairs); warps 2..9 write, 16+16 columns each
-        mbar_wait(dq_done, 0);
-        tc_fence_after();
-        if (cw < 8) {
-            const int part = (cw >> 2) & 1;
-            float v0[16], v1[16];
-            uint32_t r[16];
-            tmem_ld16(tdQ + lane_addr + part * 16, r);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; i++) v0[i] = __uint_as_float(r[i]) * p.scale;
-            tmem_ld16(tdQ + lane_addr + 32 + part * 16, r);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; i++) v1[i] = __uint_as_float(r[i]) * p.scale;
-            if (row < p.Sq) {
-                if (p.rope_cos) {
-                    const bf16* cp = p.rope_cos + (size_t)(row + off) * 32 + part * 16;
-                    const bf16* sp = p.rope_sin + (size_t)(row + off) * 32 + part * 16;
-#pragma unroll
-                    for (int i = 0; i < 16; i++) {
-                        const float c = __bfloat162float(cp[i]), sn = __bfloat162float(sp[i]);
-                        const float a = v0[i], bb = v1[i];
-                        v0[i] = a * c + bb * sn;
-                        v1[i] = bb * c - a * sn;
-                    }
-                }
-                bf16* d0 = p.dq + b * p.dq_b + (long long)row * p.dq_r + h * D + part * 16;
-                *reinterpret_cast<uint4*>(d0) = pack8(v0);
-                *reinterpret_cast<uint4*>(d0 + 8) = pack8(v0 + 8);
-                *reinterpret_cast<uint4*>(d0 + 32) = pack8(v1);
-                *reinterpret_cast<uint4*>(d0 + 40) = pack8(v1 + 8);
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
-#undef TRACE
-}
-
 // dq[rows, heads*64] (bf16, row pitch ld) = scale * (optional RoPE^T) dq_acc (fp32)
 __global__ void attn_bwd_dq_finalize_kernel(const float* __restrict__ acc, bf16* __restrict__ dq, long long rows, int W, int ld,
                                             int S, float scale, const bf16* __restrict__ rope_cos,
@@ -1912,8 +849,7 @@ __global__ void attn_bwd_dq_finalize_kernel(const float* __restrict__ acc, bf16*
 
 }   // namespace
 
-// bring-up hook: device buffer of 128 int64 receiving a clock64 trace of CTA (0,0) of the dQ kernel, or the per-phase
-// cycle sums of the forward kernel's softmax warps (NULL = off)
+// tuning hook: device buffer of 128 int64 receiving the per-phase cycle sums of the forward kernel's softmax warps (NULL = off)
 extern "C" void b200_attn_debug_trace(long long* buf) { g_attn_dbg = buf; }
 
 // defined in attn_flash.cu
@@ -1953,68 +889,29 @@ extern "C" int b200_attn_causal_bwd_tc(const void* q, const void* k, const void*
     if ((rc = tc05_make_tmap_3d(&tmK, k, W, Sk, batch, strides[4], strides[3], D, BK))) return rc;
     if ((rc = tc05_make_tmap_3d(&tmV, v, W, Sk, batch, strides[7], strides[6], D, BK))) return rc;
     if ((rc = tc05_make_tmap_3d(&tmdO, d_o, W, Sq, batch, strides[13], strides[12], D, BQ))) return rc;
+    CUtensorMap tmDQ;
+    if ((rc = tc05_make_tmap_3d_f32(&tmDQ, dq_acc, W, Sq, batch, W, (long long)Sq * W, 32, BQ))) return rc;
     BwdParams p;
-    p.lse = lse; p.delta = delta; p.dq_acc = dq_acc;
+    p.lse = lse; p.delta = delta;
     p.dk = (bf16*)dk; p.dv = (bf16*)dv;
     p.dk_b = strides[18]; p.dk_r = strides[19]; p.dv_b = strides[21]; p.dv_r = strides[22];
-    p.dqa_b = (long long)Sq * W; p.dqa_r = W;
     p.rope_cos = (const bf16*)rope_cos; p.rope_sin = (const bf16*)rope_sin;
     p.n_heads = n_heads; p.Sq = Sq; p.Sk = Sk; p.scale = scale;
-    static int dq_mode = -1;
-    if (dq_mode < 0) {
-        // B200_ATTN_BWD_DQ = tma (default): dQ tiles added into the fp32 accumulator by the TMA unit
-        //                    red          : per-lane red.global.add.v4.f32
-        //                    split        : atomic-free, dQ recomputed by a second kernel
-        const char* e = getenv("B200_ATTN_BWD_DQ");
-        dq_mode = (e && !strcmp(e, "red")) ? 1 : (e && !strcmp(e, "split")) ? 0 : 2;
-    }
     static bool configured = false;
-    static int units = 2, ldm = 0;
     if (!configured) {
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<0, 2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<1, 2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<2, 2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<2, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<2, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        // B200_ATTN_BWD_LSE = warp | direct | writer: how lse / delta reach the math warps (see the kernel's LDM parameter)
-        const char* l = getenv("B200_ATTN_BWD_LSE");
-        ldm = (l && !strcmp(l, "warp")) ? 0 : (l && !strcmp(l, "direct")) ? 1 : (l && !strcmp(l, "writer")) ? 2 : BWD_DEFAULT_LDM;
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel<2, 4, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
-        // B200_ATTN_BWD_UNITS = 2 | 4: pipeline units per query tile of the default (TMA reduce) kernel
-        const char* u = getenv("B200_ATTN_BWD_UNITS");
-        units = (u && u[0] == '2') ? 2 : (u && u[0] == '4') ? 4 : BWD_DEFAULT_UNITS;
-        B200_CUDA(cudaFuncSetAttribute(attn_bwd_dq_tc05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_DQ_BYTES), "attn_bwd_dq smem");
+        B200_CUDA(cudaFuncSetAttribute(attn_bwd_tc05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD_BYTES), "attn_bwd_tc smem");
         configured = true;
     }
+    B200_CUDA(cudaMemsetAsync(dq_acc, 0, (size_t)batch * Sq * W * sizeof(float), stream), "attn_bwd_tc memset");
     dim3 grid(batch * n_heads, (Sk + BK - 1) / BK);   // tiles on the slow index: longest first across all heads
-    if (dq_mode) {
-        CUtensorMap tmDQ;
-        if ((rc = tc05_make_tmap_3d_f32(&tmDQ, dq_acc, W, Sq, batch, W, (long long)Sq * W, 32, BQ))) return rc;
-        B200_CUDA(cudaMemsetAsync(dq_acc, 0, (size_t)batch * Sq * W * sizeof(float), stream), "attn_bwd_tc memset");
-        if (dq_mode == 2 && units == 4) attn_bwd_tc05_kernel<2, 4, 0><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
-        else if (dq_mode == 2 && ldm == 1) attn_bwd_tc05_kernel<2, 2, 1><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
-        else if (dq_mode == 2 && ldm == 2) attn_bwd_tc05_kernel<2, 2, 2><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
-        else if (dq_mode == 2) attn_bwd_tc05_kernel<2, 2, 0><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
-        else attn_bwd_tc05_kernel<1, 2, 0><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
-        B200_CHECK_LAUNCH("attn_causal_bwd_tc");
-        const long long rows = (long long)batch * Sq;
-        long long nthr = rows * (W / 16);
-        int blocks = (int)((nthr + 255) / 256);
-        if (blocks > b200_num_sms() * 16) blocks = b200_num_sms() * 16;
-        attn_bwd_dq_finalize_kernel<<<blocks, 256, 0, stream>>>(dq_acc, (bf16*)dq, rows, (int)W, (int)strides[16], Sq, scale,
-                                                                (const bf16*)rope_cos, (const bf16*)rope_sin);
-        B200_CHECK_LAUNCH("attn_bwd_dq_finalize");
-    } else {
-        attn_bwd_tc05_kernel<0, 2, 0><<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmQ, p);
-        B200_CHECK_LAUNCH("attn_causal_bwd_tc_dkv");
-        DqParams dp;
-        dp.lse = lse; dp.delta = delta; dp.dq = (bf16*)dq; dp.dq_b = strides[15]; dp.dq_r = strides[16];
-        dp.rope_cos = (const bf16*)rope_cos; dp.rope_sin = (const bf16*)rope_sin;
-        dp.n_heads = n_heads; dp.Sq = Sq; dp.Sk = Sk; dp.scale = scale;
-        dp.dbg = g_attn_dbg;
-        dim3 gq(batch * n_heads, (Sq + BQ - 1) / BQ);   // tiles on the slow index: longest first across all heads
-        attn_bwd_dq_tc05_kernel<<<gq, BWD_THREADS, SMEM_DQ_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, dp);
-        B200_CHECK_LAUNCH("attn_causal_bwd_tc_dq");
-    }
+    attn_bwd_tc05_kernel<<<grid, BWD_THREADS, SMEM_BWD_BYTES, stream>>>(tmQ, tmK, tmV, tmdO, tmDQ, p);
+    B200_CHECK_LAUNCH("attn_causal_bwd_tc");
+    const long long rows = (long long)batch * Sq;
+    long long nthr = rows * (W / 16);
+    int blocks = (int)((nthr + 255) / 256);
+    if (blocks > b200_num_sms() * 16) blocks = b200_num_sms() * 16;
+    attn_bwd_dq_finalize_kernel<<<blocks, 256, 0, stream>>>(dq_acc, (bf16*)dq, rows, (int)W, (int)strides[16], Sq, scale,
+                                                            (const bf16*)rope_cos, (const bf16*)rope_sin);
+    B200_CHECK_LAUNCH("attn_bwd_dq_finalize");
     return B200_OK;
 }

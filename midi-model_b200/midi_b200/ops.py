@@ -268,14 +268,9 @@ def _strides_packed(S: int, H: int, D: int, col0: int, ld: int):
     return [S * ld, ld, D]
 
 
-import os as _os
-
-# "tc" = tcgen05 / TMEM / TMA kernel (csrc/attn_tc05.cu); "mma" = mma.sync kernel (csrc/attn_flash.cu)
-ATTN_FWD_IMPL = _os.environ.get("B200_ATTN_FWD", "tc")
-ATTN_BWD_IMPL = _os.environ.get("B200_ATTN_BWD", "tc")
-
-
-def attn_causal_fwd(qkv: torch.Tensor, B: int, S: int, n_heads: int, D: int, want_lse: bool, impl: Optional[str] = None):
+# impl: "tc" = tcgen05 / TMEM / TMA kernels (csrc/attn_tc05.cu); "mma" = mma.sync kernels (csrc/attn_flash.cu), the reference
+# the tc kernels are tested against
+def attn_causal_fwd(qkv: torch.Tensor, B: int, S: int, n_heads: int, D: int, want_lse: bool, impl: str = "tc"):
     """qkv: [B*S, 3H] packed post-RoPE -> out [B*S, H], lse [B, h, S] fp32."""
     H = n_heads * D
     ld = qkv.stride(0)
@@ -283,16 +278,16 @@ def attn_causal_fwd(qkv: torch.Tensor, B: int, S: int, n_heads: int, D: int, wan
     lse = torch.empty((B, n_heads, S), dtype=torch.float32, device=qkv.device) if want_lse else None
     st = torch.tensor([S * ld, ld, D] * 3 + [S * H, H, D], dtype=torch.int64)
     base = qkv.data_ptr()
-    fn = "b200_attn_causal_fwd_tc" if (impl or ATTN_FWD_IMPL) == "tc" else "b200_attn_causal_fwd"
+    fn = "b200_attn_causal_fwd_tc" if impl == "tc" else "b200_attn_causal_fwd"
     lib.call(fn, base, base + 2 * H, base + 4 * H, out.data_ptr(), lib.ptr(lse), st.data_ptr(), B,
              n_heads, S, S, D, 1.0 / math.sqrt(D), lib.stream())
     return out, lse
 
 
 def attn_causal_bwd(qkv: torch.Tensor, out: torch.Tensor, dout: torch.Tensor, lse: torch.Tensor, B: int, S: int,
-                    n_heads: int, D: int, rope=None, impl: Optional[str] = None) -> torch.Tensor:
+                    n_heads: int, D: int, rope=None, impl: str = "tc") -> torch.Tensor:
     """`rope=(cos, sin)`: also apply the RoPE backward to dq, dk (gradient w.r.t. the pre-rotation projections)."""
-    if (impl or ATTN_BWD_IMPL) == "tc":
+    if impl == "tc":
         return _attn_causal_bwd_tc(qkv, out, dout, lse, B, S, n_heads, D, rope)
     H = n_heads * D
     ld = qkv.stride(0)

@@ -197,24 +197,26 @@ def _sdpa_ref(q, k, v, off):
 
 
 def check_attn_flash():
+    """Both attention implementations, forward (output and lse) and backward, directly against fp32 autograd."""
     out = {}
-    for (B, S, nh) in ((2, 64, 4), (1, 200, 16), (2, 2047, 16)):
-        D, H = 64, nh * 64
-        qkv = randn(B * S, 3 * H, seed=S)
-        o, lse = ops.attn_causal_fwd(qkv, B, S, nh, D, want_lse=True)
-        q32 = qkv.float().view(B, S, 3, nh, D).permute(2, 0, 3, 1, 4).clone().requires_grad_(True)
-        ref = _sdpa_ref(q32[0], q32[1], q32[2], 0)
-        out[f"flash_fwd_S{S}"] = rel(o.float().view(B, S, nh, D).transpose(1, 2), ref)
-        sc = (q32[0] @ q32[1].transpose(-1, -2)) / 8.0
-        msk = torch.triu(torch.ones(S, S, device=DEV, dtype=torch.bool), 1)
-        out[f"flash_lse_S{S}"] = rel(lse, torch.logsumexp(sc.masked_fill(msk, float("-inf")), -1))
-        do = randn(B * S, H, seed=S + 1)
-        dqkv = ops.attn_causal_bwd(qkv, o, do, lse, B, S, nh, D)
-        ref.backward(do.float().view(B, S, nh, D).transpose(1, 2))
-        g = q32.grad.permute(1, 3, 0, 2, 4).reshape(B * S, 3 * H)
-        out[f"flash_bwd_dq_S{S}"] = rel(dqkv[:, :H].float(), g[:, :H])
-        out[f"flash_bwd_dk_S{S}"] = rel(dqkv[:, H:2 * H].float(), g[:, H:2 * H])
-        out[f"flash_bwd_dv_S{S}"] = rel(dqkv[:, 2 * H:].float(), g[:, 2 * H:])
+    for impl in ("tc", "mma"):
+        for (B, S, nh) in ((2, 64, 4), (1, 200, 16), (2, 2047, 16)):
+            D, H = 64, nh * 64
+            qkv = randn(B * S, 3 * H, seed=S)
+            o, lse = ops.attn_causal_fwd(qkv, B, S, nh, D, want_lse=True, impl=impl)
+            q32 = qkv.float().view(B, S, 3, nh, D).permute(2, 0, 3, 1, 4).clone().requires_grad_(True)
+            ref = _sdpa_ref(q32[0], q32[1], q32[2], 0)
+            out[f"flash_fwd_S{S}_{impl}"] = rel(o.float().view(B, S, nh, D).transpose(1, 2), ref)
+            sc = (q32[0] @ q32[1].transpose(-1, -2)) / 8.0
+            msk = torch.triu(torch.ones(S, S, device=DEV, dtype=torch.bool), 1)
+            out[f"flash_lse_S{S}_{impl}"] = rel(lse, torch.logsumexp(sc.masked_fill(msk, float("-inf")), -1))
+            do = randn(B * S, H, seed=S + 1)
+            dqkv = ops.attn_causal_bwd(qkv, o, do, lse, B, S, nh, D, impl=impl)
+            ref.backward(do.float().view(B, S, nh, D).transpose(1, 2))
+            g = q32.grad.permute(1, 3, 0, 2, 4).reshape(B * S, 3 * H)
+            out[f"flash_bwd_dq_S{S}_{impl}"] = rel(dqkv[:, :H].float(), g[:, :H])
+            out[f"flash_bwd_dk_S{S}_{impl}"] = rel(dqkv[:, H:2 * H].float(), g[:, H:2 * H])
+            out[f"flash_bwd_dv_S{S}_{impl}"] = rel(dqkv[:, 2 * H:].float(), g[:, 2 * H:])
     return out
 
 

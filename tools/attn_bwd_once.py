@@ -1,5 +1,4 @@
-"""Launch the event-level attention backward a few times at the bench shape (B=8, S=2048, 16 heads, d=64): ncu target.
-B200_ATTN_BWD_DQ=tma|red|split selects the dQ path."""
+"""Launch the event-level attention backward a few times at the bench shape (B=8, S=2048, 16 heads, d=64): ncu target."""
 import os
 import sys
 
@@ -23,4 +22,4 @@ for _ in range(10):
     ops.attn_causal_bwd(qkv, o, do, lse, B, S, nh, D, impl="tc")
 e1.record()
 torch.cuda.synchronize()
-print("mode", os.environ.get("B200_ATTN_BWD_DQ", "tma"), "ms per backward", e0.elapsed_time(e1) / 10, float(dqkv.float().abs().mean()))
+print("ms per backward", e0.elapsed_time(e1) / 10, float(dqkv.float().abs().mean()))
